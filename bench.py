@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — allocation decisions/sec of the best-fit path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl native|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl native|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic requests: score R
 requests against the node's capacity table, write R device indices, the per-device
@@ -59,6 +59,7 @@ REPLAYS = int(os.environ.get("EGPU_BENCH_REPLAYS", "101"))
 USE_GATE = [not os.environ.get("EGPU_BENCH_NO_GATE")]
 GATE_NOTE = [None]
 RING = 32  # batches in the rotation: 32 x 12 MB (1M rows) = 384 MB > 126 MB L2
+DUMP_ROWS = 1 << 22  # --dump-outputs: batches of up to this many rows are written whole
 
 
 def peaks():
@@ -170,6 +171,30 @@ class ClockSampler:
                 "samples": len(self.sm), "how": self.how}
 
 
+def output_arrays(idx, delta=None, table_out=None):
+    """What the last timed step handed its caller, as floats that hold every value exactly: indices
+    (-1..63) and table' in float32 / float64, demand sums (< 2**53) in float64.  The indices of a batch
+    of more than DUMP_ROWS rows are a fixed, seeded sample of rows, stored with their row numbers
+    (at most 48 MB together)."""
+    out = {}
+    if idx.size > DUMP_ROWS:
+        rows = np.unique(np.random.default_rng(0).integers(0, idx.size, DUMP_ROWS))
+        out["indices_rows"] = rows.astype(np.float64)
+        idx = idx[rows]
+    out["indices"] = idx.astype(np.float32)
+    if delta is not None:
+        out["delta"] = delta.astype(np.float64)          # int64[2*D]: core sums, then mem sums
+    if table_out is not None:
+        out["table_out"] = table_out.astype(np.float64)  # int32[3*D]: free_core', free_mem', oversub
+    return out
+
+
+def write_outputs(out_dir, arrays, suffix=""):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}{suffix}.npy"), a)
+
+
 def make_host_batches(e, w, rank, nb, R):
     return [e.synth.requests(w["dist"], w["seed"], R, first_row=(rank * nb + b) * R) for b in range(nb)]
 
@@ -233,6 +258,8 @@ def run_reference(args, w, e, rank, world):
         rc, rm = batches[i % len(batches)]
         oracle_c.snapshot_into(fc, fm, rc, rm, idx, threads)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, output_arrays(idx))
     val = args.steps * R / dt
     line = {
         "impl": "reference", "metric": METRIC, "value": val, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
@@ -392,7 +419,12 @@ def main():
                          "(peer-fused, EGPU_F_APPLY); or NCCL all-gather + apply_deltas")
     ap.add_argument("--force-peer", action="store_true", help="experiment: the sharded step structure even at N = 1 (exchange with self)")
     ap.add_argument("--cpu-budget", type=float, default=3.0, help="seconds per CPU-baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (float32 / float64; inputs are seeded, so two "
+                         "builds can be compared output for output); with N > 1 every rank writes <name>_rank<r>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
 
     # stdout carries exactly one JSON line: whatever libraries print there (NCCL prints its
@@ -507,6 +539,9 @@ def main():
         return timed_replays(torch, dist, alloc, stream, g, world, dev, REPLAYS), counts[0]
 
     ms_list, launches = measure(leg)
+    if args.dump_outputs:  # every replay of the region rewrites the same ring entries with the same values
+        _, _, d_idx, d_delta, d_table = leg.ring[(K - 1) % nb]
+        dump = output_arrays(d_idx.cpu().numpy(), d_delta.cpu().numpy(), d_table.cpu().numpy())
     timing = summarise(ms_list, K)
     ms = timing["ms_per_step_median"] * K
     value = world * R * K / (ms * 1e-3)
@@ -874,6 +909,8 @@ def main():
         print(json.dumps(line), flush=True)
         os.dup2(2, 1)
 
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, dump, f"_rank{rank}" if world > 1 else "")
     alloc.close()
     if world > 1:
         dist.destroy_process_group()

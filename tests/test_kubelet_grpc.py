@@ -122,11 +122,14 @@ def conversation(stub, T, oracle_c, resource):
     assert ei.value.code() == grpc.StatusCode.UNKNOWN
 
 
-def serve_and_talk(tmp_path, handle, lib, oracle_c, resource=CORE):
+def serve_and_talk(tmp_path, monkeypatch, handle, lib, oracle_c, resource=CORE):
     import grpc
     from elastic_gpu_agent_b200 import kubelet_plugin as kp
     T = kp.messages()
-    sock = f"unix://{tmp_path}/elastic-gpushare-core.sock"      # pkg/plugins/base.go:226
+    # the socket is named relative to tmp_path: a unix socket path holds at most 107 bytes, and a deep
+    # temporary directory alone can be longer than that
+    monkeypatch.chdir(tmp_path)
+    sock = "unix:elastic-gpushare-core.sock"      # pkg/plugins/base.go:226
     server = grpc.server(futures.ThreadPoolExecutor(max_workers=4))
     kp.add_to_server(kp.BestFitDevicePlugin(handle, resource, lib), server)
     server.add_insecure_port(sock)
@@ -153,7 +156,7 @@ def test_wire_format_matches_the_v1beta1_field_numbers():
     assert resp.SerializeToString() == b"\x0a\x042-75"
 
 
-def test_fake_kubelet_round_trip_on_cpu_harness(tmp_path, oracle_c):
+def test_fake_kubelet_round_trip_on_cpu_harness(tmp_path, monkeypatch, oracle_c):
     os.makedirs(os.path.dirname(SO), exist_ok=True)
     cmd = ["/usr/bin/g++", "-std=c++17", "-O1", "-Wall", "-Werror", "-shared", "-fPIC", "-I", os.path.join(ROOT, "include"),
            os.path.join(ROOT, "elastic-gpu-agent_b200", "csrc", "egpu_plugin.cc"), os.path.join(HERE, "plugin_host_harness.cc"), "-o", SO]
@@ -165,15 +168,15 @@ def test_fake_kubelet_round_trip_on_cpu_harness(tmp_path, oracle_c):
     cb = cb_t(lambda fc, fm, D, core, mem: pick(C.c_void_p(fc), C.c_void_p(fm), D, core, mem))
     lib.stub_use_callback(cb)
     try:
-        serve_and_talk(tmp_path, C.c_void_p(1), lib, oracle_c)
+        serve_and_talk(tmp_path, monkeypatch, C.c_void_p(1), lib, oracle_c)
     finally:
         lib.stub_use_callback(cb_t())
 
 
 @pytest.mark.gpu
-def test_fake_kubelet_round_trip_on_gpu(tmp_path, alloc, oracle_c, egpu):
+def test_fake_kubelet_round_trip_on_gpu(tmp_path, monkeypatch, alloc, oracle_c, egpu):
     # the context also tracks a committed table: the RPCs must leave it alone
     alloc.set_table([100, 40, 75], [183359, 9000, 50000])
-    serve_and_talk(tmp_path, alloc.handle, egpu.load(), oracle_c)
+    serve_and_talk(tmp_path, monkeypatch, alloc.handle, egpu.load(), oracle_c)
     fc, fm, ov = alloc.table()
     assert fc.tolist() == [100, 40, 75] and fm.tolist() == [183359, 9000, 50000] and not ov.any()
