@@ -35,23 +35,6 @@ namespace {
 
 constexpr int64_t kMaxRows = (1ll << 31) - 1;  // EGPU_MAX_ROWS
 
-template <int DT, int THREADS>
-SnapLaunch make_launch(bool grid_variant) {
-    SnapLaunch l;
-    l.fn = grid_variant ? bestfit_grid_kernel<DT, THREADS> : bestfit_sorted_kernel<DT, THREADS>;
-    l.threads = THREADS;
-    l.smem = sizeof(SnapSmem<DT, THREADS>);
-    l.ctas_per_sm = 0;
-    return l;
-}
-
-SnapLaunch pick_launch(int D, bool grid_variant) {
-    if (D <= 8) return make_launch<8, 256>(grid_variant);
-    if (D <= 16) return make_launch<16, 256>(grid_variant);
-    if (D <= 32) return make_launch<32, 256>(grid_variant);
-    return make_launch<64, 128>(grid_variant);
-}
-
 // host copy of resort_table_cta: sorted view of a freshly set table
 void fill_sorted(DevState& h) {
     const int D = h.D;
@@ -75,6 +58,14 @@ void fill_sorted(DevState& h) {
 }
 
 // ---- output ranges of the launches in flight (pipelined launches must not share outputs) ----
+// the three outputs of one batch: indices, demand sums, table'
+void batch_outputs(egpu_ctx::Range* r, const void* idx, int64_t R, const void* delta, const void* table_out, int D) {
+    const uintptr_t pi = reinterpret_cast<uintptr_t>(idx), pd = reinterpret_cast<uintptr_t>(delta),
+                    pt = reinterpret_cast<uintptr_t>(table_out);
+    r[0] = {pi, pi + static_cast<uintptr_t>(R) * sizeof(int32_t)};
+    r[1] = {pd, pd + (pd ? sizeof(long long) * 2 * D : 0)};
+    r[2] = {pt, pt + (pt ? sizeof(int32_t) * 3 * D : 0)};
+}
 // `r[0..n)`: drops empty ranges, sorts by address; returns the new count, or -1 when two of
 // them overlap each other.
 int prepare_ranges(egpu_ctx::Range* r, int n) {
@@ -109,83 +100,100 @@ void new_group(egpu_ctx* ctx) {
     ctx->inflight.clear();
 }
 
-// first use of a kernel on this context: opt in to its shared-memory size, ask occupancy
-int configure_launch(egpu_ctx* ctx, SnapLaunch& l, int D, bool grid_variant, bool lut_variant, bool contig) {
-    if (l.ctas_per_sm != 0) return EGPU_OK;
-    const int bucket = D <= 8 ? 0 : D <= 16 ? 1 : D <= 32 ? 2 : 3;
+// ---- the scan kernels ----
+int d_bucket(int D) { return D <= 8 ? 0 : D <= 16 ? 1 : D <= 32 ? 2 : 3; }
+
+// Every scan kernel of one D bucket.  The register scans run 256 threads per CTA (128 at D = 64),
+// the lookup scans 256 whatever D is.
+template <int DT, int THREADS = (DT == 64 ? 128 : 256)>
+void fill_bucket(egpu_ctx* ctx, int b) {
+    using Snap = SnapSmem<DT, THREADS>;
+    using Lut = LutSmem<256>;
+    ctx->single[kSorted][b] = {bestfit_sorted_kernel<DT, THREADS>, THREADS, sizeof(Snap)};
+    ctx->single[kGrid][b] = {bestfit_grid_kernel<DT, THREADS>, THREADS, sizeof(Snap)};
+    ctx->single[kLut][b] = {bestfit_lut_kernel<256>, 256, sizeof(Lut)};
+    ctx->single[kSortedContig][b] = {bestfit_sorted_kernel<DT, THREADS, true>, THREADS, sizeof(Snap)};
+    ctx->single[kLutContig][b] = {bestfit_lut_kernel<256, true>, 256, sizeof(Lut)};
+    ctx->multi[0][b] = {bestfit_sorted_multi_kernel<DT, THREADS>, THREADS, sizeof(Snap)};
+    ctx->multi[1][b] = {bestfit_lut_multi_kernel<256>, 256, sizeof(Lut)};
+    ctx->packed[b] = {bestfit_sorted_packed_kernel<DT, THREADS>, THREADS, sizeof(Snap)};
+}
+
+// first use of a kernel on this context: opt in to its shared-memory size, ask its occupancy
+template <class Fn>
+int configure(egpu_ctx* ctx, ScanKernel<Fn>& k) {
+    if (k.ctas_per_sm != 0) return EGPU_OK;
     int per_sm = 0;
-    if (lut_variant) {
-        l.threads = 256;
-        l.lut_fn = contig ? bestfit_lut_kernel<256, true> : bestfit_lut_kernel<256, false>;
-        l.smem = sizeof(LutSmem<256>);
-        EGPU_CUDA(ctx, cudaFuncSetAttribute(l.lut_fn, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(l.smem)));
-        EGPU_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, l.lut_fn, l.threads, l.smem));
-    } else {
-        l = pick_launch(D, grid_variant);
-        if (!grid_variant && !contig && bucket == 0 && ctx->threads8 != 256)  // experiment knob: CTA size of the D <= 8 scan
-            l = ctx->threads8 == 128 ? make_launch<8, 128>(false) : make_launch<8, 512>(false);
-        if (contig) {
-            l.fn = bucket == 0 ? bestfit_sorted_kernel<8, 256, true> : bucket == 1 ? bestfit_sorted_kernel<16, 256, true>
-                   : bucket == 2 ? bestfit_sorted_kernel<32, 256, true> : bestfit_sorted_kernel<64, 128, true>;
-        }
-        EGPU_CUDA(ctx, cudaFuncSetAttribute(l.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(l.smem)));
-        EGPU_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, l.fn, l.threads, l.smem));
-    }
-    l.ctas_per_sm = per_sm < 1 ? 1 : per_sm;
+    EGPU_CUDA(ctx, cudaFuncSetAttribute(k.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(k.smem)));
+    EGPU_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k.fn, k.threads, k.smem));
+    k.ctas_per_sm = per_sm < 1 ? 1 : per_sm;
     return EGPU_OK;
 }
 
-// user_flags: EGPU_F_COMMIT | EGPU_F_INPUTS_READY.  finalize = 0 only for the
-// chunked host pipeline (accumulate demand sums across launches).
-int launch_snapshot(egpu_ctx* ctx, const int32_t* d_rc, const int32_t* d_rm, int64_t R, int32_t* d_idx,
-                    long long* d_delta, int32_t* d_table_out, int user_flags, bool finalize, cudaStream_t s,
-                    int rpt_hint = 0, unsigned long long push_step_plus1 = 0, bool contig = false, int* n_tiles_out = nullptr,
-                    int lag = 0) {
-    if (R > kMaxRows) return EGPU_ERR_INVALID;  // the scans index 128-bit vectors with 32 bits
-    const bool grid_variant = ctx->variant == EGPU_VARIANT_GRID;
-    const bool lut_variant = ctx->variant == EGPU_VARIANT_LUT || (ctx->variant == EGPU_VARIANT_AUTO && ctx->D > 16);
-    const int bucket = ctx->D <= 8 ? 0 : ctx->D <= 16 ? 1 : ctx->D <= 32 ? 2 : 3;
-    if (contig && grid_variant) return EGPU_ERR_STATE;  // the literal variant has no prefix-commit mode
-    SnapLaunch& l = ctx->snap[contig ? (lut_variant ? 4 : 3) : grid_variant ? 1 : (lut_variant ? 2 : 0)][bucket];
-    {
-        const int rc = configure_launch(ctx, l, ctx->D, grid_variant, lut_variant, contig);
-        if (rc != EGPU_OK) return rc;
-    }
-    if (lut_variant && ctx->lut_dirty) {  // refresh the lookup tables on the launching stream
-        lut_build_kernel<<<1, 256, 0, s>>>(ctx->d_state, ctx->d_lut);
-        EGPU_CUDA(ctx, cudaGetLastError());
-        ctx->launches += 1;
-        ctx->lut_dirty = false;
-        ctx->prev_is_scan = false;
-    }
-    int flags = (finalize ? kFlagFinalize : 0) | ((user_flags & EGPU_F_COMMIT) ? kFlagCommit : 0);
-    // Programmatic dependent launch.  Every scan carries the PDL attribute, so the
-    // hardware may schedule it while its predecessor is still running.  A fully
-    // ordered launch waits (griddepcontrol.wait) before it touches anything.  A
-    // pipelined launch (kFlagLateWait) runs scan and epilogue at once — its epilogue
-    // state is its own slot — and waits only before exiting.  That is allowed when
-    //  - the caller vouches its inputs were complete before the previous launch on
-    //    this stream (EGPU_F_INPUTS_READY),
-    //  - the previous launch was a scan of this context on the same stream that
-    //    does not rewrite the table, and this one is a plain finalising scan,
-    //  - it does not commit (a committing launch rewrites the table the launches still in
-    //    flight read and compute their table' from: it is always fully ordered),
-    //  - its outputs (indices, demand sums, table') are disjoint from the outputs
-    //    of every launch since the last fully ordered one, and
-    //  - fewer than pipe_group launches have been issued since then, which bounds
-    //    the launches in flight to pipe_group + 1 < kEpiSlots.
-    egpu_ctx::Range mine[3] = {
-        {reinterpret_cast<uintptr_t>(d_idx), reinterpret_cast<uintptr_t>(d_idx) + static_cast<uintptr_t>(R) * sizeof(int32_t)},
-        {reinterpret_cast<uintptr_t>(d_delta), reinterpret_cast<uintptr_t>(d_delta) + (d_delta ? sizeof(long long) * 2 * ctx->D : 0)},
-        {reinterpret_cast<uintptr_t>(d_table_out), reinterpret_cast<uintptr_t>(d_table_out) + (d_table_out ? sizeof(int32_t) * 3 * ctx->D : 0)}};
-    const int n_mine = prepare_ranges(mine, 3);
-    if (n_mine < 0) return EGPU_ERR_INVALID;  // two of this launch's own outputs overlap
-    bool pipelined = !grid_variant && !contig && finalize && (user_flags & EGPU_F_INPUTS_READY) && !(user_flags & EGPU_F_COMMIT) &&
-                     ctx->prev_is_scan && !ctx->prev_changes_table && ctx->prev_stream == s && ctx->group_len > 0 &&
-                     !overlaps_inflight(ctx->inflight, mine, n_mine);
+// A scan launch with the programmatic-dependent-launch attribute (see pdl_flags).
+template <class... Params, class... Args>
+int launch_pdl(egpu_ctx* ctx, const ScanKernel<void (*)(Params...)>& k, int64_t ctas, cudaStream_t s, const Args&... args) {
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cudaLaunchConfig_t cfg{};
+    cfg.gridDim = dim3(static_cast<unsigned>(ctas));
+    cfg.blockDim = dim3(static_cast<unsigned>(k.threads));
+    cfg.dynamicSmemBytes = k.smem;
+    cfg.stream = s;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    EGPU_CUDA(ctx, cudaLaunchKernelEx(&cfg, k.fn, args...));
+    ctx->launches += 1;
+    return EGPU_OK;
+}
+
+bool uses_lut(const egpu_ctx* ctx) {
+    return ctx->variant == EGPU_VARIANT_LUT || (ctx->variant == EGPU_VARIANT_AUTO && ctx->D > 16);
+}
+
+// rebuild the lookup tables on the launching stream when the table has changed since they were built
+int refresh_lut(egpu_ctx* ctx, cudaStream_t s) {
+    if (!ctx->lut_dirty) return EGPU_OK;
+    lut_build_kernel<<<1, 256, 0, s>>>(ctx->d_state, ctx->d_lut);
+    EGPU_CUDA(ctx, cudaGetLastError());
+    ctx->launches += 1;
+    ctx->lut_dirty = false;
+    ctx->prev_is_scan = false;
+    return EGPU_OK;
+}
+
+// Launches per pipelined group.  With a ring of 32 output buffers, groups of 24 with boundary
+// launches give 2.34 us per step against 2.45 for groups of 16 (B200, DESIGN.md 7.2).
+constexpr int kPipeGroup = 24;
+static_assert(kPipeGroup + 1 < kEpiSlots, "every launch in flight needs its own epilogue slot");
+
+// Programmatic dependent launch.  Every scan carries the PDL attribute, so the
+// hardware may schedule it while its predecessor is still running.  A fully
+// ordered launch waits (griddepcontrol.wait) before it touches anything.  A
+// pipelined launch (kFlagLateWait) runs scan and epilogue at once — its epilogue
+// state is its own slot — and waits only before exiting.  That is allowed when
+//  - the caller vouches its inputs were complete before the previous launch on
+//    this stream (EGPU_F_INPUTS_READY),
+//  - the previous launch was a scan of this context on the same stream that
+//    does not rewrite the table, and this one is a plain scan (`may_pipeline`),
+//  - it does not commit (a committing launch rewrites the table the launches still in
+//    flight read and compute their table' from: it is always fully ordered),
+//  - its outputs (indices, demand sums, table') are disjoint from the outputs
+//    of every launch since the last fully ordered one, and
+//  - fewer than kPipeGroup launches have been issued since then, which bounds
+//    the launches in flight to kPipeGroup + 1 < kEpiSlots, and the epi_multi slots
+//    they hold (`mbatches` more for this launch) to half of that ring.
+// Returns the launch's PDL flags; starts a new group unless the launch pipelines.
+int pdl_flags(egpu_ctx* ctx, bool may_pipeline, int user_flags, cudaStream_t s, const egpu_ctx::Range* mine, int n_mine,
+              int mbatches) {
+    const bool pipelined = may_pipeline && (user_flags & EGPU_F_INPUTS_READY) && !(user_flags & EGPU_F_COMMIT) &&
+                           ctx->prev_is_scan && !ctx->prev_changes_table && ctx->prev_stream == s && ctx->group_len > 0 &&
+                           !overlaps_inflight(ctx->inflight, mine, n_mine);
+    int flags = 0;
     if (pipelined) {
         flags |= kFlagLateWait;
-        if (ctx->group_len >= ctx->pipe_group) {
+        if (ctx->group_len >= kPipeGroup || ctx->group_mbatches + mbatches > kMultiSlots - kMultiMax) {
             // group boundary: this launch still scans alongside its predecessors, but it waits
             // for them before its epilogue and only then lets its successors start; it becomes
             // the first member of the next group
@@ -200,45 +208,68 @@ int launch_snapshot(egpu_ctx* ctx, const int32_t* d_rc, const int32_t* d_rm, int
     // (Checked on B200, scripts/probes/pdl_event_probe.cu and scripts/eager_probe.py: events
     // and ordinary kernels enqueued after a PDL launch still wait for its completion.)
     if (user_flags & EGPU_F_INPUTS_READY) flags |= kFlagEarlyTrigger;
-    const unsigned long long slot = (finalize ? (ctx->seq % kEpiSlots) : static_cast<unsigned long long>(kEpiSlots)) |
-                                    (push_step_plus1 << 8) | (static_cast<unsigned long long>(lag) << 56);
+    return flags;
+}
 
-    // Grid: one resident wave at most.  A lone launch wants every SM pulling at once
-    // (8 rows per thread, one trip); launches of a pipelined stream overlap each
-    // other, so a smaller grid with more rows per thread (48) costs fewer CTA
-    // launches, fewer atomics and leaves room for the neighbours — measured best on
-    // B200 at R = 1M.  The zero-copy path passes its own hint (see egpu_bestfit_batch).
-    const int64_t nvec = R >> 2;
-    int rpt = 8;
-    // (measured and dropped: giving the launches of a pipelined stream that could not themselves be
-    // pipelined - the first of a graph - the lone-launch grid: 2.80 against 2.68 us per step)
-    if (user_flags & EGPU_F_INPUTS_READY) rpt = (lut_variant || ctx->D <= 16) ? 48 : 8;  // measured, scripts/tune_*.sh
-    else if (lut_variant) rpt = 32;  // the lookup scan has a 13 KB per-CTA table tile to amortise
+// after a scan launch that went through pdl_flags: it joins the group, and the next scan may pipeline behind it
+void note_scan(egpu_ctx* ctx, cudaStream_t s, const egpu_ctx::Range* mine, int n_mine, bool commit, int mbatches) {
+    add_inflight(ctx, mine, n_mine);
+    ctx->group_len += 1;
+    ctx->group_mbatches += mbatches;
+    ctx->prev_is_scan = true;
+    ctx->prev_changes_table = commit;
+    ctx->prev_stream = s;
+    if (commit) ctx->lut_dirty = true;
+}
+
+// Grid of a single-batch launch: one resident wave at most.  A lone launch wants every SM pulling
+// at once (8 rows per thread, one trip); launches of a pipelined stream overlap each other, so a
+// smaller grid with more rows per thread (48) costs fewer CTA launches, fewer atomics and leaves
+// room for the neighbours — measured best on B200 at R = 1M.  A lone lookup scan has a 13 KB
+// per-CTA table tile to amortise (32).  The zero-copy path passes its own hint (see egpu_bestfit_batch).
+// (Measured and dropped: giving the launches of a pipelined stream that could not themselves be
+// pipelined - the first of a graph - the lone-launch grid: 2.80 against 2.68 us per step.)
+constexpr int kRowsPerThread = 8;
+constexpr int kRowsPerThreadPipelined = 48;  // lookup scan or D <= 16
+constexpr int kRowsPerThreadLoneLut = 32;
+// Batches this large get two waves of CTAs: the CTA scheduler then evens out the SMs (see launch_multi).
+constexpr int64_t kTwoWaveRows = 16ll << 20;
+
+// One batch.  user_flags: EGPU_F_COMMIT | EGPU_F_INPUTS_READY.
+int launch_snapshot(egpu_ctx* ctx, const int32_t* d_rc, const int32_t* d_rm, int64_t R, int32_t* d_idx,
+                    long long* d_delta, int32_t* d_table_out, int user_flags, cudaStream_t s,
+                    int rpt_hint = 0, unsigned long long push_step_plus1 = 0, bool contig = false, int* n_tiles_out = nullptr,
+                    int lag = 0) {
+    if (R > kMaxRows) return EGPU_ERR_INVALID;  // the scans index 128-bit vectors with 32 bits
+    const bool grid_variant = ctx->variant == EGPU_VARIANT_GRID;
+    const bool lut = uses_lut(ctx);
+    if (contig && grid_variant) return EGPU_ERR_STATE;  // the literal variant has no prefix-commit mode
+    ScanKernel<SingleFn>& kern =
+        ctx->single[contig ? (lut ? kLutContig : kSortedContig) : grid_variant ? kGrid : (lut ? kLut : kSorted)][d_bucket(ctx->D)];
+    int rc = configure(ctx, kern);
+    if (rc == EGPU_OK && lut) rc = refresh_lut(ctx, s);
+    if (rc != EGPU_OK) return rc;
+    egpu_ctx::Range mine[3];
+    batch_outputs(mine, d_idx, R, d_delta, d_table_out, ctx->D);
+    const int n_mine = prepare_ranges(mine, 3);
+    if (n_mine < 0) return EGPU_ERR_INVALID;  // two of this launch's own outputs overlap
+    const bool commit = (user_flags & EGPU_F_COMMIT) != 0;
+    const int flags = kFlagFinalize | (commit ? kFlagCommit : 0) | pdl_flags(ctx, !grid_variant && !contig, user_flags, s, mine, n_mine, 0);
+    const unsigned long long slot = (ctx->seq % kEpiSlots) | (push_step_plus1 << 8) | (static_cast<unsigned long long>(lag) << 56);
+
+    int rpt = kRowsPerThread;
+    if (user_flags & EGPU_F_INPUTS_READY) rpt = (lut || ctx->D <= 16) ? kRowsPerThreadPipelined : kRowsPerThread;
+    else if (lut) rpt = kRowsPerThreadLoneLut;
     if (rpt_hint > 0) rpt = rpt_hint;
-    if (ctx->rows_per_thread > 0) rpt = ctx->rows_per_thread;
     if (grid_variant) rpt = 4;
-    const int64_t per_cta = static_cast<int64_t>(l.threads) * ((rpt + 3) / 4);
-    int64_t want = (nvec + per_cta - 1) / per_cta;
-    int per_sm = l.ctas_per_sm;
-    if (ctx->ctas_per_sm_cap > 0 && ctx->ctas_per_sm_cap < per_sm) per_sm = ctx->ctas_per_sm_cap;
-    // one resident wave; two for a huge batch (the CTA scheduler then evens out the SMs, see launch_multi)
-    const int64_t cap = static_cast<int64_t>(ctx->sm_count) * per_sm * ((R >= (16ll << 20) && !contig) ? 2 : 1);
+    const int64_t per_cta = static_cast<int64_t>(kern.threads) * ((rpt + 3) / 4);
+    int64_t want = ((R >> 2) + per_cta - 1) / per_cta;
+    const int64_t cap = static_cast<int64_t>(ctx->sm_count) * kern.ctas_per_sm * ((R >= kTwoWaveRows && !contig) ? 2 : 1);
     if (want > cap) want = cap;
     if (want < 1) want = 1;
     // lane-private sums hold 2^19 rows per lane (kAccShift): keep rows/thread below that
-    const int64_t rows_per_thread = R / (want * l.threads) + 8;
-    if (rows_per_thread >= (1ll << 19)) return EGPU_ERR_INVALID;
+    if (R / (want * kern.threads) + 8 >= (1ll << 19)) return EGPU_ERR_INVALID;
 
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3(static_cast<unsigned>(want));
-    cfg.blockDim = dim3(static_cast<unsigned>(l.threads));
-    cfg.dynamicSmemBytes = l.smem;
-    cfg.stream = s;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
     unsigned long long* tile_sums = nullptr;
     if (contig) {  // one tile per CTA: make room for their sums
         if (want > ctx->tile_cap) {
@@ -251,62 +282,29 @@ int launch_snapshot(egpu_ctx* ctx, const int32_t* d_rc, const int32_t* d_rm, int
         tile_sums = ctx->d_tile_sums;
         if (n_tiles_out) *n_tiles_out = static_cast<int>(want);
     }
-    if (lut_variant)
-        EGPU_CUDA(ctx, cudaLaunchKernelEx(&cfg, l.lut_fn, ctx->d_state, d_rc, d_rm, static_cast<long long>(R), d_idx,
-                                          d_delta, d_table_out, flags, slot, static_cast<const DevLut*>(ctx->d_lut), tile_sums));
-    else
-        EGPU_CUDA(ctx, cudaLaunchKernelEx(&cfg, l.fn, ctx->d_state, d_rc, d_rm, static_cast<long long>(R), d_idx,
-                                          d_delta, d_table_out, flags, slot, tile_sums));
-    if (flags & kFlagCommit) ctx->lut_dirty = true;
-    ctx->launches += 1;
+    rc = launch_pdl(ctx, kern, want, s, ctx->d_state, d_rc, d_rm, static_cast<long long>(R), d_idx, d_delta, d_table_out, flags,
+                    slot, static_cast<const DevLut*>(ctx->d_lut), tile_sums);
+    if (rc != EGPU_OK) return rc;
     ctx->seq += 1;
-    add_inflight(ctx, mine, n_mine);
-    ctx->group_len += 1;
-    ctx->prev_is_scan = finalize;
-    ctx->prev_changes_table = (flags & kFlagCommit) != 0;
-    ctx->prev_stream = s;
+    note_scan(ctx, s, mine, n_mine, commit, 0);
     return EGPU_OK;
 }
 
+// Multi-batch grids: enough CTAs per batch that a thread has at least this many rows.
+constexpr int kMultiRowsPerThread = 8;
+
 // Multi-batch launch: K batches, all scored against the current table, one grid (CTA (b, t) =
 // tile t of batch b), one epilogue slot per batch.  Pipelines behind its predecessor under the
-// same conditions as launch_snapshot; a launch group never holds more than half of the
+// same conditions as a single-batch launch; a launch group never holds more than half of the
 // epi_multi ring, so the slots of everything that can be in flight are distinct.
 // push_base = first exchange step + 1 when every batch also pushes its demand vector to the peers.
 int launch_multi(egpu_ctx* ctx, const egpu_batch* bs, int K, int user_flags, cudaStream_t s, unsigned long long push_base) {
     if (ctx->variant == EGPU_VARIANT_GRID) return EGPU_ERR_STATE;  // the literal variant has no multi-batch form
-    const bool lut_variant = ctx->variant == EGPU_VARIANT_LUT || (ctx->variant == EGPU_VARIANT_AUTO && ctx->D > 16);
-    const int bucket = ctx->D <= 8 ? 0 : ctx->D <= 16 ? 1 : ctx->D <= 32 ? 2 : 3;
-    MultiLaunch& l = ctx->multi[lut_variant ? 1 : 0][bucket];
-    if (l.ctas_per_sm == 0) {
-        int per_sm = 0;
-        if (lut_variant) {
-            l.lut_fn = bestfit_lut_multi_kernel<256>;
-            l.threads = 256;
-            l.smem = sizeof(LutSmem<256>);
-            EGPU_CUDA(ctx, cudaFuncSetAttribute(l.lut_fn, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(l.smem)));
-            EGPU_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, l.lut_fn, l.threads, l.smem));
-        } else {
-            static const SortedMultiKernel fns[4] = {bestfit_sorted_multi_kernel<8, 256>, bestfit_sorted_multi_kernel<16, 256>,
-                                                     bestfit_sorted_multi_kernel<32, 256>, bestfit_sorted_multi_kernel<64, 128>};
-            static const int threads[4] = {256, 256, 256, 128};
-            static const size_t smem[4] = {sizeof(SnapSmem<8, 256>), sizeof(SnapSmem<16, 256>), sizeof(SnapSmem<32, 256>),
-                                           sizeof(SnapSmem<64, 128>)};
-            l.fn = fns[bucket];
-            l.threads = threads[bucket];
-            l.smem = smem[bucket];
-            EGPU_CUDA(ctx, cudaFuncSetAttribute(l.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(l.smem)));
-            EGPU_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, l.fn, l.threads, l.smem));
-        }
-        l.ctas_per_sm = per_sm < 1 ? 1 : per_sm;
-    }
-    if (lut_variant && ctx->lut_dirty) {
-        lut_build_kernel<<<1, 256, 0, s>>>(ctx->d_state, ctx->d_lut);
-        EGPU_CUDA(ctx, cudaGetLastError());
-        ctx->launches += 1;
-        ctx->lut_dirty = false;
-        ctx->prev_is_scan = false;
-    }
+    const bool lut = uses_lut(ctx);
+    ScanKernel<MultiFn>& kern = ctx->multi[lut ? 1 : 0][d_bucket(ctx->D)];
+    int rc = configure(ctx, kern);
+    if (rc == EGPU_OK && lut) rc = refresh_lut(ctx, s);
+    if (rc != EGPU_OK) return rc;
     MultiArgs args;
     std::memset(&args, 0, sizeof args);
     egpu_ctx::Range* mine = ctx->multi_ranges;
@@ -321,41 +319,21 @@ int launch_multi(egpu_ctx* ctx, const egpu_batch* bs, int K, int user_flags, cud
         args.b[k].table_out = (push_base && !(user_flags & EGPU_F_APPLY)) ? nullptr : b.d_table_out;
         args.b[k].R = b.R;
         if (b.R > max_r) max_r = b.R;
-        const uintptr_t pi = reinterpret_cast<uintptr_t>(b.d_out_idx), pd = reinterpret_cast<uintptr_t>(b.d_delta),
-                        pt = reinterpret_cast<uintptr_t>(args.b[k].table_out);
-        mine[3 * k] = {pi, pi + static_cast<uintptr_t>(b.R) * sizeof(int32_t)};
-        mine[3 * k + 1] = {pd, pd + (pd ? sizeof(long long) * 2 * ctx->D : 0)};
-        mine[3 * k + 2] = {pt, pt + (pt ? sizeof(int32_t) * 3 * ctx->D : 0)};
+        batch_outputs(mine + 3 * k, b.d_out_idx, b.R, b.d_delta, args.b[k].table_out, ctx->D);
     }
     const int n_mine = prepare_ranges(mine, 3 * K);
     if (n_mine < 0) return EGPU_ERR_INVALID;  // two batches of one launch share an output: their order would be undefined
-    int flags = kFlagFinalize | ((push_base && (user_flags & EGPU_F_APPLY)) ? kFlagApplyNow : 0);
-    bool pipelined = (user_flags & EGPU_F_INPUTS_READY) && ctx->prev_is_scan && !ctx->prev_changes_table && ctx->prev_stream == s &&
-                     ctx->group_len > 0 && !overlaps_inflight(ctx->inflight, mine, n_mine);
-    if (pipelined) {
-        flags |= kFlagLateWait;
-        if (ctx->group_len >= ctx->pipe_group || ctx->group_mbatches + K > kMultiSlots - kMultiMax) {
-            flags |= kFlagBoundary;
-            new_group(ctx);
-        }
-    } else {
-        new_group(ctx);
-    }
-    if (user_flags & EGPU_F_INPUTS_READY) flags |= kFlagEarlyTrigger;
+    const int flags = kFlagFinalize | ((push_base && (user_flags & EGPU_F_APPLY)) ? kFlagApplyNow : 0) | pdl_flags(ctx, true, user_flags, s, mine, n_mine, K);
 
-    // tiles per batch: enough CTAs that a thread has >= multi_rpt rows, at most the resident
+    // tiles per batch: enough CTAs that a thread has >= kMultiRowsPerThread rows, at most the resident
     // capacity of the GPU shared out among the K batches
-    const int64_t nvec = max_r >> 2;
-    const int64_t per_cta = static_cast<int64_t>(l.threads) * ((ctx->multi_rpt + 3) / 4);
-    int64_t tiles = (nvec + per_cta - 1) / per_cta;
+    const int64_t per_cta = static_cast<int64_t>(kern.threads) * ((kMultiRowsPerThread + 3) / 4);
+    int64_t tiles = ((max_r >> 2) + per_cta - 1) / per_cta;
     if (tiles < 1) tiles = 1;
-    int per_sm = l.ctas_per_sm;
-    if (ctx->ctas_per_sm_cap > 0 && ctx->ctas_per_sm_cap < per_sm) per_sm = ctx->ctas_per_sm_cap;
     // CTAs resident at once, x waves.  One wave is best for 1 M-row batches (every extra CTA is an extra
     // epilogue); for a few huge batches two waves of half-size CTAs let the hardware's CTA scheduler even
-    // out the SMs (64 Mi rows: 129 -> 124 us per batch, same-box A/B with EGPU_MULTI_WAVES)
-    const int waves = ctx->multi_waves > 0 ? ctx->multi_waves : (max_r >= (16ll << 20) ? 2 : 1);
-    const int64_t cap = static_cast<int64_t>(ctx->sm_count) * per_sm * waves;
+    // out the SMs (64 Mi rows: 129 -> 124 us per batch, same-box A/B)
+    const int64_t cap = static_cast<int64_t>(ctx->sm_count) * kern.ctas_per_sm * (max_r >= kTwoWaveRows ? 2 : 1);
     int64_t extra = 0;
     if (tiles * K > cap) {  // capped: hand the resident CTAs out evenly, the first `extra` batches get one more
         tiles = cap / K;
@@ -366,34 +344,14 @@ int launch_multi(egpu_ctx* ctx, const egpu_batch* bs, int K, int user_flags, cud
         }
     }
     if (tiles > 0xffff) tiles = 0xffff;
-    if (max_r / (tiles * l.threads) + 8 >= (1ll << 19)) return EGPU_ERR_INVALID;  // lane-private sums hold 2^19 rows per lane
+    if (max_r / (tiles * kern.threads) + 8 >= (1ll << 19)) return EGPU_ERR_INVALID;  // lane-private sums hold 2^19 rows per lane
     const int tiles_extra = static_cast<int>(tiles | (extra << 16));
-    const int64_t n_ctas = tiles * K + extra;
-
     const unsigned int slot_base = static_cast<unsigned int>(ctx->mseq % kMultiSlots);
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3(static_cast<unsigned>(n_ctas));
-    cfg.blockDim = dim3(static_cast<unsigned>(l.threads));
-    cfg.dynamicSmemBytes = l.smem;
-    cfg.stream = s;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    if (lut_variant)
-        EGPU_CUDA(ctx, cudaLaunchKernelEx(&cfg, l.lut_fn, ctx->d_state, args, tiles_extra, flags, slot_base, push_base,
-                                          static_cast<const DevLut*>(ctx->d_lut)));
-    else
-        EGPU_CUDA(ctx, cudaLaunchKernelEx(&cfg, l.fn, ctx->d_state, args, tiles_extra, flags, slot_base, push_base));
-    ctx->launches += 1;
+    rc = launch_pdl(ctx, kern, tiles * K + extra, s, ctx->d_state, args, tiles_extra, flags, slot_base, push_base,
+                    static_cast<const DevLut*>(ctx->d_lut));
+    if (rc != EGPU_OK) return rc;
     ctx->mseq += static_cast<uint64_t>(K);
-    add_inflight(ctx, mine, n_mine);
-    ctx->group_len += 1;
-    ctx->group_mbatches += K;
-    ctx->prev_is_scan = true;
-    ctx->prev_changes_table = false;
-    ctx->prev_stream = s;
+    note_scan(ctx, s, mine, n_mine, false, K);
     return EGPU_OK;
 }
 
@@ -404,7 +362,7 @@ int launch_prefix_commit(egpu_ctx* ctx, const int32_t* d_rc, const int32_t* d_rm
     if (!ctx->d_prefix_out) EGPU_CUDA(ctx, cudaMalloc(&ctx->d_prefix_out, sizeof(PrefixOut) + sizeof(long long) * 2 * kMaxD));
     int n_tiles = 0;
     // the scan itself must neither publish nor commit: its sums are the uncapped ones
-    int rc = launch_snapshot(ctx, d_rc, d_rm, R, d_idx, nullptr, nullptr, 0, true, s, 0, 0, true, &n_tiles);
+    int rc = launch_snapshot(ctx, d_rc, d_rm, R, d_idx, nullptr, nullptr, 0, s, 0, 0, true, &n_tiles);
     if (rc != EGPU_OK) return rc;
     PrefixOut* pf = static_cast<PrefixOut*>(ctx->d_prefix_out);
     prefix_cut_kernel<<<ctx->D, 256, 0, s>>>(ctx->d_state, d_idx, d_rc, d_rm, R, n_tiles, ctx->d_tile_sums, pf);
@@ -512,7 +470,7 @@ int launch_prefix_commit_shard(egpu_ctx* ctx, const int32_t* d_rc, const int32_t
     long long* base = reinterpret_cast<long long*>(pf + 1);
     int n_tiles = 0;
     // finalising scan without commit: its epilogue publishes (and pushes) the uncapped sums
-    int rc = launch_snapshot(ctx, d_rc, d_rm, R, d_idx, nullptr, nullptr, 0, true, s, 0, step + 1, true, &n_tiles);
+    int rc = launch_snapshot(ctx, d_rc, d_rm, R, d_idx, nullptr, nullptr, 0, s, 0, step + 1, true, &n_tiles);
     if (rc != EGPU_OK) return rc;
     prefix_base_kernel<<<1, kMaxD, 0, s>>>(ctx->d_state, step + 1, base);
     prefix_cut_kernel<<<ctx->D, 256, 0, s>>>(ctx->d_state, d_idx, d_rc, d_rm, R, n_tiles, ctx->d_tile_sums, pf, base);
@@ -532,50 +490,27 @@ int launch_prefix_commit_shard(egpu_ctx* ctx, const int32_t* d_rc, const int32_t
     return EGPU_OK;
 }
 
-using PackedKernel = void (*)(DevState*, const uint32_t*, long long, signed char*, long long*, int32_t*, int, unsigned long long);
-
 // Packed-format scan: always a fully ordered launch (it serves the synchronous host path).
 int launch_packed(egpu_ctx* ctx, const uint32_t* d_req, int64_t R, signed char* d_idx8, long long* d_delta,
                   int32_t* d_table_out, int user_flags, cudaStream_t s, int rows_per_thread) {
-    const int bucket = ctx->D <= 8 ? 0 : ctx->D <= 16 ? 1 : ctx->D <= 32 ? 2 : 3;
-    static const PackedKernel fns[4] = {bestfit_sorted_packed_kernel<8, 256>, bestfit_sorted_packed_kernel<16, 256>,
-                                        bestfit_sorted_packed_kernel<32, 256>, bestfit_sorted_packed_kernel<64, 128>};
-    static const int threads[4] = {256, 256, 256, 128};
-    static const size_t smem[4] = {sizeof(SnapSmem<8, 256>), sizeof(SnapSmem<16, 256>), sizeof(SnapSmem<32, 256>),
-                                   sizeof(SnapSmem<64, 128>)};
-    int& per_sm = ctx->packed_ctas_per_sm[bucket];
-    if (per_sm == 0) {
-        EGPU_CUDA(ctx, cudaFuncSetAttribute(fns[bucket], cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem[bucket])));
-        int n = 0;
-        EGPU_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, fns[bucket], threads[bucket], smem[bucket]));
-        per_sm = n < 1 ? 1 : n;
-    }
+    ScanKernel<PackedFn>& kern = ctx->packed[d_bucket(ctx->D)];
+    int rc = configure(ctx, kern);
+    if (rc != EGPU_OK) return rc;
     const int64_t nchunk = R >> 9;  // 512 requests per warp trip
-    const int64_t per_cta = static_cast<int64_t>(threads[bucket] / 32) * ((rows_per_thread + 15) / 16);
+    const int64_t per_cta = static_cast<int64_t>(kern.threads / 32) * ((rows_per_thread + 15) / 16);
     int64_t want = (nchunk + per_cta - 1) / per_cta;
-    const int64_t cap = static_cast<int64_t>(ctx->sm_count) * per_sm;
+    const int64_t cap = static_cast<int64_t>(ctx->sm_count) * kern.ctas_per_sm;
     if (want > cap) want = cap;
     if (want < 1) want = 1;
-    if (R / (want * threads[bucket]) + 16 >= (1ll << 19)) return EGPU_ERR_INVALID;
-    const int flags = kFlagFinalize | ((user_flags & EGPU_F_COMMIT) ? kFlagCommit : 0);
-    const unsigned long long slot = ctx->seq % kEpiSlots;
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3(static_cast<unsigned>(want));
-    cfg.blockDim = dim3(static_cast<unsigned>(threads[bucket]));
-    cfg.dynamicSmemBytes = smem[bucket];
-    cfg.stream = s;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    EGPU_CUDA(ctx, cudaLaunchKernelEx(&cfg, fns[bucket], ctx->d_state, d_req, static_cast<long long>(R), d_idx8, d_delta,
-                                      d_table_out, flags, slot));
-    ctx->launches += 1;
+    if (R / (want * kern.threads) + 16 >= (1ll << 19)) return EGPU_ERR_INVALID;
+    const bool commit = (user_flags & EGPU_F_COMMIT) != 0;
+    rc = launch_pdl(ctx, kern, want, s, ctx->d_state, d_req, static_cast<long long>(R), d_idx8, d_delta, d_table_out,
+                    kFlagFinalize | (commit ? kFlagCommit : 0), static_cast<unsigned long long>(ctx->seq % kEpiSlots));
+    if (rc != EGPU_OK) return rc;
     ctx->seq += 1;
     new_group(ctx);
     ctx->prev_is_scan = false;  // the int32 scans do not pipeline behind this one
-    if (flags & kFlagCommit) ctx->lut_dirty = true;
+    if (commit) ctx->lut_dirty = true;
     return EGPU_OK;
 }
 
@@ -641,25 +576,15 @@ int egpu_ctx_create(int cuda_device, egpu_ctx** out) {
     egpu_ctx* ctx = new (std::nothrow) egpu_ctx();
     if (!ctx) return EGPU_ERR_NOMEM;
     ctx->dev = cuda_device;
+    fill_bucket<8>(ctx, 0);
+    fill_bucket<16>(ctx, 1);
+    fill_bucket<32>(ctx, 2);
+    fill_bucket<64>(ctx, 3);
     int rc = [&]() -> int {
         EGPU_CUDA(ctx, cudaSetDevice(cuda_device));
         cudaDeviceProp prop;
         EGPU_CUDA(ctx, cudaGetDeviceProperties(&prop, cuda_device));
         ctx->sm_count = prop.multiProcessorCount;
-        if (const char* e = std::getenv("EGPU_CTAS_PER_SM")) ctx->ctas_per_sm_cap = std::atoi(e);
-        if (const char* e = std::getenv("EGPU_ROWS_PER_THREAD")) ctx->rows_per_thread = std::atoi(e);
-        if (const char* e = std::getenv("EGPU_REPLAY_GENERAL")) ctx->replay_general = std::atoi(e) != 0;
-        if (const char* e = std::getenv("EGPU_REPLAY_VARIANT")) ctx->replay_variant = std::atoi(e);
-        if (const char* e = std::getenv("EGPU_THREADS8")) {
-            const int v = std::atoi(e);
-            ctx->threads8 = (v == 128 || v == 512) ? v : 256;
-        }
-        if (const char* e = std::getenv("EGPU_MULTI_WAVES")) ctx->multi_waves = std::max(0, std::min(8, std::atoi(e)));
-        if (const char* e = std::getenv("EGPU_MULTI_RPT")) ctx->multi_rpt = std::max(4, std::min(4096, std::atoi(e)));
-        if (const char* e = std::getenv("EGPU_PIPE_GROUP")) {
-            const int g = std::atoi(e);
-            ctx->pipe_group = g < 1 ? 1 : (g > kPipeGroupMax ? kPipeGroupMax : g);
-        }
         EGPU_CUDA(ctx, cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking));
         EGPU_CUDA(ctx, cudaMalloc(&ctx->d_state, sizeof(DevState)));
         EGPU_CUDA(ctx, cudaMemsetAsync(ctx->d_state, 0, sizeof(DevState), ctx->stream));
@@ -670,7 +595,6 @@ int egpu_ctx_create(int cuda_device, egpu_ctx** out) {
         EGPU_CUDA(ctx, cudaMalloc(&ctx->d_table_out, sizeof(int32_t) * 3 * kMaxD));
         EGPU_CUDA(ctx, cudaMallocHost(&ctx->h_delta, sizeof(long long) * 2 * kMaxD));
         EGPU_CUDA(ctx, cudaHostGetDevicePointer(reinterpret_cast<void**>(&ctx->h_delta_dev), ctx->h_delta, 0));
-        if (const char* e = std::getenv("EGPU_NO_ZERO_COPY")) ctx->no_zero_copy = std::atoi(e) != 0;
         EGPU_CUDA(ctx, cudaMallocHost(&ctx->h_table, sizeof(int32_t) * 3 * kMaxD));
         EGPU_CUDA(ctx, cudaMallocHost(&ctx->h_qtable, offsetof(DevState, peer)));
         EGPU_CUDA(ctx, cudaMallocHost(&ctx->h_gate, sizeof(unsigned long long)));
@@ -843,7 +767,7 @@ int egpu_bestfit_batch_dev(egpu_ctx* ctx, const int32_t* d_req_core, const int32
         return launch_prefix_commit(ctx, d_req_core, d_req_mem, R, d_out_idx, reinterpret_cast<long long*>(d_delta), d_table_out,
                                     flags, s);
     return launch_snapshot(ctx, d_req_core, d_req_mem, R, d_out_idx, reinterpret_cast<long long*>(d_delta),
-                           d_table_out, flags, true, s);
+                           d_table_out, flags, s);
 }
 
 static int check_batches(const egpu_batch* batches, int32_t K) {
@@ -944,21 +868,19 @@ int egpu_bestfit_query(egpu_ctx* ctx, const int32_t* free_core, const int32_t* f
     EGPU_CUDA(ctx, cudaMemcpyAsync(ctx->d_req_core, req_core, sizeof(int32_t) * R, cudaMemcpyHostToDevice, s));
     EGPU_CUDA(ctx, cudaMemcpyAsync(ctx->d_req_mem, req_mem, sizeof(int32_t) * R, cudaMemcpyHostToDevice, s));
     // the register scan whatever the context's variant: one table, used once - lookup tables would not pay
-    const int bucket = D <= 8 ? 0 : D <= 16 ? 1 : D <= 32 ? 2 : 3;
-    SnapLaunch& l = ctx->snap[0][bucket];
-    rc = configure_launch(ctx, l, D, false, false, false);
+    ScanKernel<SingleFn>& kern = ctx->single[kSorted][d_bucket(D)];
+    rc = configure(ctx, kern);
     if (rc != EGPU_OK) return rc;
-    const int64_t nvec = R >> 2;
-    const int64_t per_cta = static_cast<int64_t>(l.threads) * 2;
-    int64_t want = (nvec + per_cta - 1) / per_cta;
-    const int64_t cap = static_cast<int64_t>(ctx->sm_count) * l.ctas_per_sm;
+    const int64_t per_cta = static_cast<int64_t>(kern.threads) * 2;
+    int64_t want = ((R >> 2) + per_cta - 1) / per_cta;
+    const int64_t cap = static_cast<int64_t>(ctx->sm_count) * kern.ctas_per_sm;
     if (want > cap) want = cap;
     if (want < 1) want = 1;
-    if (R / (want * l.threads) + 8 >= (1ll << 19)) return EGPU_ERR_INVALID;
+    if (R / (want * kern.threads) + 8 >= (1ll << 19)) return EGPU_ERR_INVALID;
     // fully ordered launch (no PDL flags), epilogue slot 0 of the scratch state, nothing published
-    l.fn<<<static_cast<unsigned>(want), l.threads, l.smem, s>>>(ctx->d_qstate, ctx->d_req_core, ctx->d_req_mem,
-                                                                static_cast<long long>(R), ctx->d_idx, nullptr, nullptr,
-                                                                kFlagFinalize, 0ull, nullptr);
+    kern.fn<<<static_cast<unsigned>(want), kern.threads, kern.smem, s>>>(ctx->d_qstate, ctx->d_req_core, ctx->d_req_mem,
+                                                                         static_cast<long long>(R), ctx->d_idx, nullptr, nullptr,
+                                                                         kFlagFinalize, 0ull, nullptr, nullptr);
     EGPU_CUDA(ctx, cudaGetLastError());
     ctx->launches += 1;
     ctx->prev_is_scan = false;
@@ -985,10 +907,10 @@ int egpu_bestfit_batch(egpu_ctx* ctx, const int32_t* req_core, const int32_t* re
     const int32_t* zm = R > 0 ? static_cast<const int32_t*>(mapped_alias(req_mem)) : nullptr;
     int32_t* zi = R > 0 ? static_cast<int32_t*>(mapped_alias(out_idx)) : nullptr;
     const bool prefix = (commit & EGPU_F_PREFIX_COMMIT) != 0;  // `commit` carries EGPU_F_COMMIT | EGPU_F_PREFIX_COMMIT
-    if (!prefix && zc && zm && zi && aligned16(zc) && aligned16(zm) && aligned16(zi) && !ctx->no_zero_copy) {
+    if (!prefix && zc && zm && zi && aligned16(zc) && aligned16(zm) && aligned16(zi)) {
         // 64 rows per thread: few CTAs, many trips, so reads of later rows and writes of
         // earlier ones are on the link at the same time (PCIe is full duplex)
-        rc = launch_snapshot(ctx, zc, zm, R, zi, ctx->h_delta_dev, nullptr, (commit & EGPU_F_COMMIT) ? EGPU_F_COMMIT : 0, true, s, 64);
+        rc = launch_snapshot(ctx, zc, zm, R, zi, ctx->h_delta_dev, nullptr, (commit & EGPU_F_COMMIT) ? EGPU_F_COMMIT : 0, s, 64);
         if (rc != EGPU_OK) return rc;
         EGPU_CUDA(ctx, cudaStreamSynchronize(s));
     } else {
@@ -1001,7 +923,7 @@ int egpu_bestfit_batch(egpu_ctx* ctx, const int32_t* req_core, const int32_t* re
         rc = prefix ? launch_prefix_commit(ctx, ctx->d_req_core, ctx->d_req_mem, R, ctx->d_idx, ctx->d_delta, nullptr,
                                            (commit & EGPU_F_COMMIT) ? EGPU_F_COMMIT : 0, s)
                     : launch_snapshot(ctx, ctx->d_req_core, ctx->d_req_mem, R, ctx->d_idx, ctx->d_delta, nullptr,
-                                      (commit & EGPU_F_COMMIT) ? EGPU_F_COMMIT : 0, true, s);
+                                      (commit & EGPU_F_COMMIT) ? EGPU_F_COMMIT : 0, s);
         if (rc != EGPU_OK) return rc;
         if (R > 0) EGPU_CUDA(ctx, cudaMemcpyAsync(out_idx, ctx->d_idx, sizeof(int32_t) * R, cudaMemcpyDeviceToHost, s));
         EGPU_CUDA(ctx, cudaMemcpyAsync(ctx->h_delta, ctx->d_delta, sizeof(long long) * 2 * D, cudaMemcpyDeviceToHost, s));
@@ -1134,7 +1056,7 @@ int egpu_bestfit_batch_shard_dev(egpu_ctx* ctx, const int32_t* d_req_core, const
     EGPU_CUDA(ctx, cudaSetDevice(ctx->dev));
     cudaStream_t s = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
     return launch_snapshot(ctx, d_req_core, d_req_mem, R, d_out_idx, reinterpret_cast<long long*>(d_delta), nullptr,
-                           flags, true, s, 0, step + 1);
+                           flags, s, 0, step + 1);
 }
 
 int egpu_bestfit_batch_shard_prefix_dev(egpu_ctx* ctx, const int32_t* d_req_core, const int32_t* d_req_mem, int64_t R,
@@ -1164,7 +1086,7 @@ int egpu_bestfit_batch_shard_lag_dev(egpu_ctx* ctx, const int32_t* d_req_core, c
     EGPU_CUDA(ctx, cudaSetDevice(ctx->dev));
     cudaStream_t s = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
     return launch_snapshot(ctx, d_req_core, d_req_mem, R, d_out_idx, reinterpret_cast<long long*>(d_delta), d_table_out_lagged,
-                           flags, true, s, 0, step + 1, false, nullptr, lag);
+                           flags, s, 0, step + 1, false, nullptr, lag);
 }
 
 int egpu_table_apply_peers_multi_dev(egpu_ctx* ctx, uint64_t first_step, int nsteps, int32_t* const* d_table_outs,
@@ -1230,7 +1152,7 @@ int egpu_bestfit_batch_packed(egpu_ctx* ctx, const uint32_t* req_packed, int64_t
     int rc;
     const uint32_t* zr = R > 0 ? static_cast<const uint32_t*>(mapped_alias(req_packed)) : nullptr;
     signed char* zi = R > 0 ? static_cast<signed char*>(mapped_alias(out_idx8)) : nullptr;
-    if (zr && zi && aligned16(zr) && aligned16(zi) && !ctx->no_zero_copy) {  // zero-copy across PCIe, see egpu_bestfit_batch
+    if (zr && zi && aligned16(zr) && aligned16(zi)) {  // zero-copy across PCIe, see egpu_bestfit_batch
         rc = launch_packed(ctx, zr, R, zi, ctx->h_delta_dev, nullptr, commit ? EGPU_F_COMMIT : 0, s, 128);
         if (rc != EGPU_OK) return rc;
         EGPU_CUDA(ctx, cudaStreamSynchronize(s));
@@ -1316,7 +1238,6 @@ int egpu_replay(egpu_ctx* ctx, const int32_t* kind, const int32_t* a, const int3
         smem = static_cast<size_t>((E + 15) & ~15ll);
         if (!ctx->replay_configured) {
             EGPU_CUDA(ctx, cudaFuncSetAttribute(replay_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kReplaySmemEvents));
-            EGPU_CUDA(ctx, cudaFuncSetAttribute(replay8_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kReplaySmemEvents));
             ctx->replay_configured = true;
         }
     }
@@ -1325,15 +1246,14 @@ int egpu_replay(egpu_ctx* ctx, const int32_t* kind, const int32_t* a, const int3
     EGPU_CUDA(ctx, cudaMemcpyAsync(d_b, b, sizeof(int32_t) * E, cudaMemcpyHostToDevice, s));
     ctx->prev_is_scan = false;
     ctx->lut_dirty = true;
-    if (ctx->D <= 32 && E <= kReplaySmemEvents && ctx->replay_variant == 2) {
-        // two warps: decode off the chain, lane = device on it (default wherever it applies)
-        const size_t smem2 = static_cast<size_t>((E + 15) & ~15ll);
+    if (ctx->D <= 32 && E <= kReplaySmemEvents) {
+        // two warps: decode off the chain, lane = device on it
         if (!ctx->replay2_configured) {
             EGPU_CUDA(ctx, cudaFuncSetAttribute(replay2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kReplaySmemEvents));
             ctx->replay2_configured = true;
         }
-        replay2_kernel<<<1, 64, smem2, s>>>(ctx->d_state, d_kind, d_a, d_b, E, d_out);
-    } else if (ctx->D <= 8 && !ctx->replay_general)
+        replay2_kernel<<<1, 64, smem, s>>>(ctx->d_state, d_kind, d_a, d_b, E, d_out);
+    } else if (ctx->D <= 8)  // only past kReplaySmemEvents events: `live` in HBM
         replay8_kernel<<<1, 32, smem, s>>>(ctx->d_state, d_kind, d_a, d_b, E, d_out, d_live);
     else
         replay_kernel<<<1, 32, smem, s>>>(ctx->d_state, d_kind, d_a, d_b, E, d_out, d_live);

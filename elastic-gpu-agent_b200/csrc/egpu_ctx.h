@@ -13,35 +13,30 @@
 
 using namespace egpu;  // internal header: the context is made of the kernels' types
 
-using SnapKernel = void (*)(egpu::DevState*, const int32_t*, const int32_t*, long long, int32_t*, long long*, int32_t*, int,
-                            unsigned long long, unsigned long long*);
+// The scans by launch shape: one batch (the register and grid scans ignore the lookup tables),
+// several batches in one grid, the packed wire format.
+using SingleFn = void (*)(DevState*, const int32_t*, const int32_t*, long long, int32_t*, long long*, int32_t*, int,
+                          unsigned long long, const DevLut*, unsigned long long*);
+using MultiFn = void (*)(DevState*, const MultiArgs, int, int, unsigned int, unsigned long long, const DevLut*);
+using PackedFn = void (*)(DevState*, const uint32_t*, long long, signed char*, long long*, int32_t*, int, unsigned long long);
 
-using LutKernel = void (*)(egpu::DevState*, const int32_t*, const int32_t*, long long, int32_t*, long long*, int32_t*, int,
-                           unsigned long long, const egpu::DevLut*, unsigned long long*);
-
-struct SnapLaunch {
-    SnapKernel fn = nullptr;
-    LutKernel lut_fn = nullptr;  // set instead of fn for the lookup-table scan
+template <class Fn>
+struct ScanKernel {
+    Fn fn = nullptr;
     int threads = 0;
     size_t smem = 0;
     int ctas_per_sm = 0;  // 0 = not configured yet on this context
 };
 
-using SortedMultiKernel = void (*)(egpu::DevState*, const egpu::MultiArgs, int, int, unsigned int, unsigned long long);
-using LutMultiKernel = void (*)(egpu::DevState*, const egpu::MultiArgs, int, int, unsigned int, unsigned long long,
-                                const egpu::DevLut*);
-struct MultiLaunch {
-    SortedMultiKernel fn = nullptr;
-    LutMultiKernel lut_fn = nullptr;
-    int threads = 0;
-    size_t smem = 0;
-    int ctas_per_sm = 0;
-};
+enum ScanForm { kSorted, kGrid, kLut, kSortedContig, kLutContig, kSingleForms };
+constexpr int kDBuckets = 4;  // D <= 8, 16, 32, 64
 
 struct egpu_ctx {
     std::mutex mu;
-    SnapLaunch snap[5][4];            // [sorted, grid, lut, sorted CONTIG, lut CONTIG][D bucket]
-    MultiLaunch multi[2][4];          // multi-batch launches: [sorted, lut][D bucket]
+    // every scan kernel by form and D bucket (egpu_ctx_create fills them, first use configures them)
+    ScanKernel<SingleFn> single[kSingleForms][kDBuckets];
+    ScanKernel<MultiFn> multi[2][kDBuckets];  // [0 = register scan, 1 = lookup scan]
+    ScanKernel<PackedFn> packed[kDBuckets];
     void* h_qtable = nullptr;         // pinned host image of that table (the part of DevState before `peer`)
     DevState* d_qstate = nullptr;     // scratch table of egpu_bestfit_query (the context's own table is not touched)
     unsigned long long* h_gate = nullptr;      // pinned: start gates the host has opened (egpu_peer_gate_open)
@@ -74,10 +69,9 @@ struct egpu_ctx {
     int32_t* d_table_out = nullptr;   // int32[3*64]
     long long* h_delta = nullptr;     // pinned
     long long* h_delta_dev = nullptr; // its device-visible alias
-    bool no_zero_copy = false;        // EGPU_NO_ZERO_COPY=1: always stage through HBM
     int32_t* h_table = nullptr;       // pinned int32[3*64]
     bool replay_configured = false;   // shared-memory opt-in of the replay kernels done
-    // bookkeeping for programmatic dependent launch (see launch_snapshot)
+    // bookkeeping for programmatic dependent launch (see pdl_flags)
     bool prev_is_scan = false;        // the last kernel this context launched was a snapshot scan ...
     bool prev_changes_table = false;  // ... and it may rewrite the table (commit)
     cudaStream_t prev_stream = nullptr;
@@ -89,17 +83,8 @@ struct egpu_ctx {
     std::vector<Range> inflight;      // output ranges of those launches, sorted by address, pairwise disjoint
     std::vector<Range> range_tmp;
     Range multi_ranges[3 * kMultiMax];  // scratch of launch_multi
-    int multi_waves = 0;              // multi-batch launches: CTA waves the grid may hold (EGPU_MULTI_WAVES; 0 = by batch size)
-    int multi_rpt = 8;                // ... and the fewest rows per thread worth a CTA (EGPU_MULTI_RPT)
-    int pipe_group = 24;              // launches per group (EGPU_PIPE_GROUP, <= kPipeGroupMax)
-    int ctas_per_sm_cap = 0;          // 0 = occupancy limit (EGPU_CTAS_PER_SM overrides)
-    int rows_per_thread = 0;          // grid sizing target (EGPU_ROWS_PER_THREAD), 0 = default
-    int packed_ctas_per_sm[4] = {0, 0, 0, 0};  // occupancy of the packed-format scan per D bucket, 0 = not asked yet
-    int threads8 = 256;               // CTA size of the D <= 8 register scan (EGPU_THREADS8 = 128 | 256 | 512)
-    int replay_variant = 2;           // 2 = two-warp kernel where it applies (EGPU_REPLAY_VARIANT=1: round 1's one-warp kernels)
     bool replay2_configured = false;
     bool sort_sets_configured = false;  // sort_sets_smem_kernel may use 128 KB of dynamic shared memory
-    bool replay_general = false;      // EGPU_REPLAY_GENERAL=1: lane = device kernel even for D <= 8 (tests)
     // grow-only device arena for multi-kernel host-buffer pipelines (egpu_devhash.cu)
     void* arena = nullptr;
     size_t arena_cap = 0;

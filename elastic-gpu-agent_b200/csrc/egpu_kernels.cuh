@@ -41,7 +41,10 @@ constexpr uint32_t kNoCand = 32u;  // "no feasible row" among 32 positions
 constexpr uint32_t kPadWord = kGuardC;
 
 // flags of the snapshot kernels
-constexpr int kFlagFinalize = 1;  // the batch's demand sums are complete after this launch: publish delta / table'
+constexpr int kFlagFinalize = 1;  // set on every launch: publish delta / table'.  The epilogue keeps testing it:
+                                  // without the test ptxas gives the D <= 8 register scan 60 registers instead
+                                  // of 48, and pipelined single launches at D = 8 run 2.56 instead of 2.36 us
+                                  // per step (B200, 1000 W)
 constexpr int kFlagCommit = 2;    // table' replaces the table
 constexpr int kFlagLateWait = 4;  // programmatic dependent launch: this launch shares nothing
                                   // with the launches in flight before it, so it triggers its
@@ -87,6 +90,10 @@ struct PeerCfg {
     int32_t world, rank;
 };
 
+constexpr int kEpiSlots = 32;      // DevState::epi, the ring of single-batch launches
+constexpr int kMultiSlots = 128;   // DevState::epi_multi
+constexpr int kMultiMax = 64;      // batches per multi-batch launch (descriptors travel as kernel parameters)
+
 struct DevState {
     int32_t free_core[kMaxD];
     int32_t free_mem[kMaxD];
@@ -109,17 +116,13 @@ struct DevState {
         unsigned int ticket;
         unsigned int pad_[3];
         unsigned int pair[kMaxD];           // plain-snapshot epilogue: the two finishers of a device meet here
-    } epi[33];
+    } epi[kEpiSlots];
     // Multi-batch launches (egpu_bestfit_batches_dev): one slot per BATCH, taken from this ring in
     // launch order; a launch group (see launch_multi) never holds more than half of it.
-    EpiSlot epi_multi[128];
+    EpiSlot epi_multi[kMultiSlots];
     unsigned long long gate_epoch;        // start gates passed so far (egpu_peer_gate_dev)
     unsigned long long gate_timeouts;     // ... of which gave up waiting (~2 s) for the host or a peer
 };
-constexpr int kEpiSlots = 32;      // ring used by pipelined launches; slot 32 = accumulate-only launches
-constexpr int kPipeGroupMax = 24;  // at most this many launches between two fully ordered ones
-constexpr int kMultiSlots = 128;   // DevState::epi_multi
-constexpr int kMultiMax = 64;      // batches per multi-batch launch (descriptors travel as kernel parameters)
 
 // One batch of a multi-batch launch: the arguments of egpu_bestfit_batch_dev, per batch.
 // plain-snapshot epilogue: bits 49..63 of a running sum count the CTAs that have added to it

@@ -47,7 +47,8 @@ __global__ void synth_requests_kernel(int dist, unsigned long long seed, long lo
 }
 
 // =============================================================================
-// Sequential mode: one warp.  D <= 8: table in registers (replay8_kernel, below the general
+// Sequential mode: one warp, for what the two-warp kernel below does not take (D > 32, or more
+// than kReplaySmemEvents events).  D <= 8: table in registers (replay8_kernel, below the general
 // one); otherwise lane = device (two per lane when D > 32)
 // =============================================================================
 //

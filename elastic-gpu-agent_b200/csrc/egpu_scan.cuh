@@ -477,7 +477,7 @@ __global__ void __launch_bounds__(THREADS)  // (forcing 5 CTAs/SM = 48 registers
 bestfit_sorted_kernel(DevState* __restrict__ st, const int32_t* __restrict__ req_core,
                       const int32_t* __restrict__ req_mem, long long R, int32_t* __restrict__ out_idx,
                       long long* __restrict__ delta_out, int32_t* __restrict__ table_out, int flags, unsigned long long slot_step,
-                      unsigned long long* __restrict__ tile_sums) {
+                      const DevLut* __restrict__ /*glut: the lookup scan's*/, unsigned long long* __restrict__ tile_sums) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     auto& s = *reinterpret_cast<SnapSmem<DT, THREADS>*>(smem_raw);
     const bool late = (flags & kFlagLateWait) != 0;
@@ -522,7 +522,7 @@ __device__ __forceinline__ void multi_cta_to_tile(int tiles_extra, int& batch, i
 template <int DT, int THREADS>
 __global__ void __launch_bounds__(THREADS)
 bestfit_sorted_multi_kernel(DevState* __restrict__ st, const __grid_constant__ MultiArgs args, int tiles_extra, int flags,
-                            unsigned int slot_base, unsigned long long push_base) {
+                            unsigned int slot_base, unsigned long long push_base, const DevLut* __restrict__ /*glut: the lookup scan's*/) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     auto& s = *reinterpret_cast<SnapSmem<DT, THREADS>*>(smem_raw);
     const bool late = (flags & kFlagLateWait) != 0;
@@ -640,6 +640,7 @@ __global__ void __launch_bounds__(THREADS)
 bestfit_grid_kernel(DevState* __restrict__ st, const int32_t* __restrict__ req_core,
                     const int32_t* __restrict__ req_mem, long long R, int32_t* __restrict__ out_idx,
                     long long* __restrict__ delta_out, int32_t* __restrict__ table_out, int flags, unsigned long long slot_step,
+                    const DevLut* __restrict__ /*glut: the lookup scan's*/,
                     unsigned long long* __restrict__ /*tile_sums: not supported by the literal variant*/) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     auto& s = *reinterpret_cast<SnapSmem<DT, THREADS>*>(smem_raw);

@@ -130,26 +130,31 @@ def test_lookup_scan_with_clustered_memory_values(alloc, oracle_c, egpu):
         assert np.array_equal(idx, o_idx) and np.array_equal(dc, o_dc) and np.array_equal(dm, o_dm)
 
 
-def test_lookup_scan_sums_survive_many_trips(oracle_c, egpu, monkeypatch):
+def test_lookup_scan_sums_survive_many_trips(alloc, egpu):
     """Every request lands on one device with the largest addends: the 32-bit shared-memory words
-    of the lookup scan must be folded before any field overflows (4 M rows on 4 CTAs: 4096 rows
-    per thread, 512 trips)."""
-    monkeypatch.setenv("EGPU_ROWS_PER_THREAD", "4096")
-    alloc = egpu.BestFitAllocator(0)
+    of the lookup scan must be folded before any field overflows.  A lone lookup launch at
+    R >= 16 Mi holds at most 148 x 8 x 2 CTAs of 256 threads, so at R = 2^28 each thread scans
+    >= 442 rows = >= 55 trips of 8; without the fold every 32 trips the 12-bit field of a copy
+    (<= 3 per add, 4 lanes x 8 rows per trip) would overflow after 42 trips.  3 GiB of HBM."""
+    import torch
     D = 64
     fc = np.full(D, 100, dtype=np.int32)
     fm = np.full(D, (1 << 18) - 1, dtype=np.int32)
     fc[1:] = np.arange(1, D) % 100  # device 0 is the only one that takes core = 100
     fc[0] = 100
     fc[1:] = np.minimum(fc[1:], 99)
-    R = 1 << 22
-    rc = np.full(R, 100, dtype=np.int32)
-    rm = np.full(R, (1 << 18) - 1, dtype=np.int32)
+    R = 1 << 28
+    c = torch.full((R,), 100, dtype=torch.int32, device="cuda")
+    m = torch.full((R,), (1 << 18) - 1, dtype=torch.int32, device="cuda")
+    idx = torch.full((R,), -9, dtype=torch.int32, device="cuda")
+    dl = torch.zeros(2 * D, dtype=torch.int64, device="cuda")
     alloc.set_variant(3)
     alloc.set_table(fc, fm)
-    idx, dc, dm = alloc.bestfit(rc, rm)
-    alloc.close()
-    assert (idx == 0).all()
+    alloc.bestfit_dev(c.data_ptr(), m.data_ptr(), R, idx.data_ptr(), dl.data_ptr(), 0, False,
+                      torch.cuda.current_stream().cuda_stream)
+    torch.cuda.synchronize()
+    assert bool((idx == 0).all())
+    dc, dm = dl[:D].cpu().numpy(), dl[D:].cpu().numpy()
     assert dc[0] == 100 * R and dm[0] == ((1 << 18) - 1) * R and not dc[1:].any() and not dm[1:].any()
 
 

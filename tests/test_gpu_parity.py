@@ -340,42 +340,43 @@ def test_replay_random(D, E, alloc, oracle_c):
     assert np.array_equal(g_c, o_fc) and np.array_equal(g_m, o_fm)
 
 
-def test_replay_all_kernels_agree(oracle_c, egpu, monkeypatch):
-    """The two-warp kernel (default, D <= 32 and events that fit shared memory), and round 1's one-warp kernels
-    behind EGPU_REPLAY_VARIANT=1: table in registers for D <= 8, lane = device (EGPU_REPLAY_GENERAL=1 forces it).
-    All must match the oracle on the same churn stream, including double frees, frees of non-ALLOC events,
-    frees of later events and unknown kinds."""
-    kind, a, b = egpu.synth.churn_events(9, 50_000)
-    kind, a, b = kind.copy(), a.copy(), b.copy()
-    rng = np.random.default_rng(3)
-    for i in rng.integers(10, kind.size, 400):     # sprinkle the odd cases in
-        r = rng.integers(0, 5)
-        if r == 0:
-            kind[i], a[i] = 1, a[i - 1] if kind[i - 1] == 1 else i - 1        # free right after / double free
-        elif r == 1:
-            kind[i], a[i] = 1, i + 5                                           # target in the future
-        elif r == 2:
-            kind[i], a[i] = 1, -3
-        elif r == 3:
-            kind[i] = 7                                                        # unknown kind
-        else:
-            kind[i], a[i], b[i] = 0, 101, 5                                    # infeasible ALLOC (then possibly freed later)
-    for D in (1, 3, 8, 9, 32, 33):
-        fc, fm = egpu.synth.table_fragmented(40 + D, D)
-        fc = np.maximum(fc, 30)
-        o_idx, o_fc, o_fm = oracle_c.replay(fc, fm, kind, a, b)
-        for variant, general in (("2", "0"), ("1", "0"), ("1", "1")):
-            monkeypatch.setenv("EGPU_REPLAY_VARIANT", variant)
-            monkeypatch.setenv("EGPU_REPLAY_GENERAL", general)
+def test_replay_all_kernels_agree(oracle_c, egpu):
+    """Every replay kernel on churn streams with the odd cases sprinkled in (double frees, frees of non-ALLOC
+    events, frees of later events, unknown kinds), against the oracle.  The input picks the kernel: the two-warp
+    kernel for D <= 32 while the events fit shared memory (E <= 200 Ki), else the one-warp kernels - table in
+    registers for D <= 8, lane = device above - with `live` in HBM past 200 Ki events."""
+    def odd_stream(E):
+        kind, a, b = egpu.synth.churn_events(9, E)
+        kind, a, b = kind.copy(), a.copy(), b.copy()
+        rng = np.random.default_rng(3)
+        for i in rng.integers(10, kind.size, 400):     # sprinkle the odd cases in
+            r = rng.integers(0, 5)
+            if r == 0:
+                kind[i], a[i] = 1, a[i - 1] if kind[i - 1] == 1 else i - 1        # free right after / double free
+            elif r == 1:
+                kind[i], a[i] = 1, i + 5                                           # target in the future
+            elif r == 2:
+                kind[i], a[i] = 1, -3
+            elif r == 3:
+                kind[i] = 7                                                        # unknown kind
+            else:
+                kind[i], a[i], b[i] = 0, 101, 5                                    # infeasible ALLOC (then possibly freed later)
+        return kind, a, b
+
+    for E, Ds in ((50_000, (1, 3, 8, 9, 32, 33)), (200 * 1024 + 1, (1, 8, 9, 32, 33))):
+        kind, a, b = odd_stream(E)
+        for D in Ds:
+            fc, fm = egpu.synth.table_fragmented(40 + D, D)
+            fc = np.maximum(fc, 30)
+            o_idx, o_fc, o_fm = oracle_c.replay(fc, fm, kind, a, b)
             with egpu.BestFitAllocator(0) as al:
                 al.set_table(fc, fm)
                 idx = al.replay(kind, a, b)
                 g_c, g_m, _ = al.table()
-            assert np.array_equal(idx, o_idx), (D, variant, general)
-            assert np.array_equal(g_c, o_fc) and np.array_equal(g_m, o_fm)
+            assert np.array_equal(idx, o_idx), (E, D)
+            assert np.array_equal(g_c, o_fc) and np.array_equal(g_m, o_fm), (E, D)
     # sizes around the 256-event ring chunks
     fc, fm = egpu.synth.table_full(8)
-    monkeypatch.setenv("EGPU_REPLAY_VARIANT", "2")
     for E in (1, 2, 255, 256, 257, 511, 512, 513, 1000):
         k2, a2, b2 = egpu.synth.churn_events(5, E)
         o_idx, o_fc, o_fm = oracle_c.replay(fc, fm, k2, a2, b2)
