@@ -186,6 +186,15 @@ class BestFitAllocator:
                                                  C.c_void_p(p_dm), 1 if commit else 0)
         self._check(rc, "egpu_bestfit_batch_packed")
 
+    def bestfit_packed_dev(self, d_req: int, R: int, d_idx8: int, d_delta: int = 0, d_table_out: int = 0,
+                           commit: bool = False, stream: int | None = None):
+        """egpu_bestfit_batch_packed_dev: packed words and int8 indices in device memory (16-byte aligned);
+        d_delta int64[2*D] and d_table_out int32[3*D] may be 0."""
+        rc = self._lib.egpu_bestfit_batch_packed_dev(self._h, C.c_void_p(d_req), int(R), C.c_void_p(d_idx8),
+                                                     C.c_void_p(d_delta or None), C.c_void_p(d_table_out or None),
+                                                     L.F_COMMIT if commit else 0, _stream(stream))
+        self._check(rc, "egpu_bestfit_batch_packed_dev")
+
     def host_alloc(self, nbytes: int) -> int:
         p = C.c_void_p()
         self._check(self._lib.egpu_host_alloc(self._h, C.byref(p), int(nbytes)), "egpu_host_alloc")

@@ -1129,7 +1129,8 @@ int64_t egpu_peer_last_timeout(egpu_ctx* ctx) {
 
 int egpu_bestfit_batch_packed_dev(egpu_ctx* ctx, const uint32_t* d_req_packed, int64_t R, int8_t* d_out_idx8,
                                   int64_t* d_delta, int32_t* d_table_out, int flags, void* stream) {
-    if (!ctx || R < 0) return EGPU_ERR_INVALID;
+    // the epilogue's demand sums share their word with an arrival count: they hold EGPU_MAX_ROWS rows at most
+    if (!ctx || R < 0 || R > kMaxRows) return EGPU_ERR_INVALID;
     if (R > 0 && (!d_req_packed || !d_out_idx8)) return EGPU_ERR_INVALID;
     if (!aligned16(d_req_packed) || !aligned16(d_out_idx8)) return EGPU_ERR_INVALID;
     std::lock_guard<std::mutex> g(ctx->mu);
@@ -1142,7 +1143,7 @@ int egpu_bestfit_batch_packed_dev(egpu_ctx* ctx, const uint32_t* d_req_packed, i
 
 int egpu_bestfit_batch_packed(egpu_ctx* ctx, const uint32_t* req_packed, int64_t R, int8_t* out_idx8,
                               int64_t* out_delta_core, int64_t* out_delta_mem, int commit) {
-    if (!ctx || R < 0) return EGPU_ERR_INVALID;
+    if (!ctx || R < 0 || R > kMaxRows) return EGPU_ERR_INVALID;  // as egpu_bestfit_batch_packed_dev
     if (R > 0 && (!req_packed || !out_idx8)) return EGPU_ERR_INVALID;
     std::lock_guard<std::mutex> g(ctx->mu);
     if (!ctx->has_table) return EGPU_ERR_NO_TABLE;

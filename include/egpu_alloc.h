@@ -190,7 +190,9 @@ int egpu_bestfit_batch_rounds_dev(egpu_ctx* ctx, const int32_t* d_req_core,
 /* Packed wire format, for callers bound by PCIe rather than by the scan: 5 bytes per decision
  * instead of 12.  req_packed[r] = EGPU_PACK_REQUEST(core, mem) (core in 0..127, mem in
  * 0..2^18-1; any word >= 2^25, e.g. EGPU_PACKED_INVALID, is an infeasible request);
- * out_idx8[r] = device index 0..63 or -1.  Everything else as egpu_bestfit_batch. */
+ * out_idx8[r] = device index 0..63 or -1.  R <= EGPU_MAX_ROWS as in every other entry point
+ * (EGPU_ERR_INVALID above it: the demand sums hold that many rows).  Everything else as
+ * egpu_bestfit_batch. */
 #define EGPU_PACK_REQUEST(core, mem) (((uint32_t)(core) << 18) | (uint32_t)(mem))
 #define EGPU_PACKED_INVALID 0xFFFFFFFFu
 int egpu_bestfit_batch_packed(egpu_ctx* ctx, const uint32_t* req_packed, int64_t R, int8_t* out_idx8,
