@@ -99,6 +99,9 @@ def load() -> C.CDLL:
         "egpu_table_apply_deltas_dev": (C.c_int, [vp, vp, C.c_int, vp, C.c_int, vp]),
         "egpu_synth_requests_dev": (C.c_int, [vp, C.c_int, C.c_uint64, C.c_int64, C.c_int64, vp, vp, vp]),
         "egpu_replay": (C.c_int, [vp, vp, vp, vp, C.c_int64, vp]),
+        "egpu_bestfit_cards": (C.c_int, [vp, vp, vp, C.c_int64, vp, vp, vp, vp, C.c_int]),
+        "egpu_bestfit_cards_dev": (C.c_int, [vp, vp, vp, C.c_int64, vp, vp, vp, vp, C.c_int, vp]),
+        "egpu_replay_cards": (C.c_int, [vp, vp, vp, vp, C.c_int64, vp, vp]),
         "egpu_peer_export": (C.c_int, [vp, vp]),
         "egpu_peer_attach": (C.c_int, [vp, C.c_int, C.c_int, vp]),
         "egpu_peer_detach": (C.c_int, [vp]),

@@ -218,6 +218,37 @@ class BestFitAllocator:
         buf = (C.c_char * (max(1, n) * dt.itemsize)).from_address(addr)
         return np.frombuffer(buf, dtype=dt, count=n)
 
+    # -- whole-card requests (core = 100 * k asks for k whole cards) -------------
+    def bestfit_cards(self, req_core, req_mem, commit: bool = False, cards: bool = True):
+        """egpu_bestfit_cards.  Returns (idx int32[R], cards uint64[R] or None, delta_core int64[D],
+        delta_mem int64[D]); cards=False asks for no masks."""
+        rc_, rm_ = _i32(req_core), _i32(req_mem)
+        if rc_.shape != rm_.shape or rc_.ndim != 1:
+            raise L.EgpuError(L.ERR_INVALID, "bestfit_cards")
+        D = self._lib.egpu_table_size(self._h)
+        if D < 0:
+            raise L.EgpuError(D, "egpu_table_size")
+        R = rc_.size
+        idx = np.empty(R, dtype=np.int32)
+        masks = np.empty(R, dtype=np.uint64) if cards else None
+        dc = np.zeros(D, dtype=np.int64)
+        dm = np.zeros(D, dtype=np.int64)
+        rc = self._lib.egpu_bestfit_cards(self._h, _ptr(rc_), _ptr(rm_), R, _ptr(idx),
+                                          _ptr(masks) if cards else C.c_void_p(None), _ptr(dc), _ptr(dm),
+                                          L.F_COMMIT if commit else 0)
+        self._check(rc, "egpu_bestfit_cards")
+        return idx, masks, dc, dm
+
+    def bestfit_cards_dev(self, d_core: int, d_mem: int, R: int, d_idx: int, d_cards: int = 0, d_delta: int = 0,
+                          d_table_out: int = 0, commit: bool = False, stream: int | None = None, inputs_ready: bool = False):
+        """egpu_bestfit_cards_dev: device arrays (16-byte aligned); d_cards uint64[R], d_delta int64[2*D] and
+        d_table_out int32[3*D] may be 0."""
+        flags = (L.F_COMMIT if commit else 0) | (L.F_INPUTS_READY if inputs_ready else 0)
+        rc = self._lib.egpu_bestfit_cards_dev(self._h, C.c_void_p(d_core), C.c_void_p(d_mem), int(R), C.c_void_p(d_idx),
+                                              C.c_void_p(d_cards or None), C.c_void_p(d_delta or None),
+                                              C.c_void_p(d_table_out or None), flags, _stream(stream))
+        self._check(rc, "egpu_bestfit_cards_dev")
+
     # -- snapshot mode, device buffers ---------------------------------------
     def bestfit_dev(self, d_core: int, d_mem: int, R: int, d_idx: int, d_delta: int = 0, d_table_out: int = 0,
                     commit: bool = False, stream: int | None = None, inputs_ready: bool = False, prefix_commit: bool = False):
@@ -353,3 +384,15 @@ class BestFitAllocator:
         rc = self._lib.egpu_replay(self._h, _ptr(k), _ptr(a_), _ptr(b_), k.size, _ptr(out))
         self._check(rc, "egpu_replay")
         return out
+
+    def replay_cards(self, kind, a, b, cards: bool = True):
+        """egpu_replay_cards: replay with whole-card ALLOCs.  Returns (idx int32[E], cards uint64[E] or None)."""
+        k, a_, b_ = _i32(kind), _i32(a), _i32(b)
+        if not (k.shape == a_.shape == b_.shape) or k.ndim != 1:
+            raise L.EgpuError(L.ERR_INVALID, "replay_cards")
+        out = np.empty(k.size, dtype=np.int32)
+        masks = np.empty(k.size, dtype=np.uint64) if cards else None
+        rc = self._lib.egpu_replay_cards(self._h, _ptr(k), _ptr(a_), _ptr(b_), k.size, _ptr(out),
+                                         _ptr(masks) if cards else C.c_void_p(None))
+        self._check(rc, "egpu_replay_cards")
+        return out, masks

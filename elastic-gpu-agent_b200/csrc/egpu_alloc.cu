@@ -23,6 +23,7 @@
 
 #include "egpu_scan.cuh"
 #include "egpu_replay.cuh"
+#include "egpu_cards.cuh"
 
 // =============================================================================
 // Host side: context + C ABI
@@ -117,6 +118,7 @@ void fill_bucket(egpu_ctx* ctx, int b) {
     ctx->multi[0][b] = {bestfit_sorted_multi_kernel<DT, THREADS>, THREADS, sizeof(Snap)};
     ctx->multi[1][b] = {bestfit_lut_multi_kernel<256>, 256, sizeof(Lut)};
     ctx->packed[b] = {bestfit_sorted_packed_kernel<DT, THREADS>, THREADS, sizeof(Snap)};
+    ctx->cards[b] = {cards_scan_kernel<DT, THREADS>, THREADS, sizeof(CardsSmem<DT, THREADS>)};
 }
 
 // first use of a kernel on this context: opt in to its shared-memory size, ask its occupancy
@@ -235,6 +237,20 @@ constexpr int kRowsPerThreadLoneLut = 32;
 // Batches this large get two waves of CTAs: the CTA scheduler then evens out the SMs (see launch_multi).
 constexpr int64_t kTwoWaveRows = 16ll << 20;
 
+// CTAs of a single-batch launch with `rpt` rows per thread: at most one resident wave, two for
+// batches of kTwoWaveRows rows and more when `two_waves`.  0 when a lane would sum 2^19 rows or
+// more: its lane-private demand sums (kAccShift) would overflow.
+template <class Fn>
+int64_t single_ctas(const egpu_ctx* ctx, const ScanKernel<Fn>& kern, int64_t R, int rpt, bool two_waves) {
+    const int64_t per_cta = static_cast<int64_t>(kern.threads) * ((rpt + 3) / 4);
+    int64_t want = ((R >> 2) + per_cta - 1) / per_cta;
+    const int64_t cap = static_cast<int64_t>(ctx->sm_count) * kern.ctas_per_sm * ((R >= kTwoWaveRows && two_waves) ? 2 : 1);
+    if (want > cap) want = cap;
+    if (want < 1) want = 1;
+    if (R / (want * kern.threads) + 8 >= (1ll << 19)) return 0;
+    return want;
+}
+
 // One batch.  user_flags: EGPU_F_COMMIT | EGPU_F_INPUTS_READY.
 int launch_snapshot(egpu_ctx* ctx, const int32_t* d_rc, const int32_t* d_rm, int64_t R, int32_t* d_idx,
                     long long* d_delta, int32_t* d_table_out, int user_flags, cudaStream_t s,
@@ -262,13 +278,8 @@ int launch_snapshot(egpu_ctx* ctx, const int32_t* d_rc, const int32_t* d_rm, int
     else if (lut) rpt = kRowsPerThreadLoneLut;
     if (rpt_hint > 0) rpt = rpt_hint;
     if (grid_variant) rpt = 4;
-    const int64_t per_cta = static_cast<int64_t>(kern.threads) * ((rpt + 3) / 4);
-    int64_t want = ((R >> 2) + per_cta - 1) / per_cta;
-    const int64_t cap = static_cast<int64_t>(ctx->sm_count) * kern.ctas_per_sm * ((R >= kTwoWaveRows && !contig) ? 2 : 1);
-    if (want > cap) want = cap;
-    if (want < 1) want = 1;
-    // lane-private sums hold 2^19 rows per lane (kAccShift): keep rows/thread below that
-    if (R / (want * kern.threads) + 8 >= (1ll << 19)) return EGPU_ERR_INVALID;
+    const int64_t want = single_ctas(ctx, kern, R, rpt, !contig);
+    if (want == 0) return EGPU_ERR_INVALID;
 
     unsigned long long* tile_sums = nullptr;
     if (contig) {  // one tile per CTA: make room for their sums
@@ -284,6 +295,33 @@ int launch_snapshot(egpu_ctx* ctx, const int32_t* d_rc, const int32_t* d_rm, int
     }
     rc = launch_pdl(ctx, kern, want, s, ctx->d_state, d_rc, d_rm, static_cast<long long>(R), d_idx, d_delta, d_table_out, flags,
                     slot, static_cast<const DevLut*>(ctx->d_lut), tile_sums);
+    if (rc != EGPU_OK) return rc;
+    ctx->seq += 1;
+    note_scan(ctx, s, mine, n_mine, commit, 0);
+    return EGPU_OK;
+}
+
+// One batch of whole-card rows (spec 2.8): the register scan whatever the context's variant, pipelined,
+// committed and ordered with the other scans under the same rules (pdl_flags, note_scan).  d_cards
+// may be nullptr.  user_flags: EGPU_F_COMMIT | EGPU_F_INPUTS_READY.
+int launch_cards(egpu_ctx* ctx, const int32_t* d_rc, const int32_t* d_rm, int64_t R, int32_t* d_idx,
+                 unsigned long long* d_cards, long long* d_delta, int32_t* d_table_out, int user_flags, cudaStream_t s) {
+    ScanKernel<CardsFn>& kern = ctx->cards[d_bucket(ctx->D)];
+    int rc = configure(ctx, kern);
+    if (rc != EGPU_OK) return rc;
+    egpu_ctx::Range mine[4];
+    batch_outputs(mine, d_idx, R, d_delta, d_table_out, ctx->D);
+    const uintptr_t pc = reinterpret_cast<uintptr_t>(d_cards);
+    mine[3] = {pc, pc + (pc ? sizeof(unsigned long long) * static_cast<uintptr_t>(R) : 0)};
+    const int n_mine = prepare_ranges(mine, 4);
+    if (n_mine < 0) return EGPU_ERR_INVALID;  // two of this launch's own outputs overlap
+    const bool commit = (user_flags & EGPU_F_COMMIT) != 0;
+    const int flags = kFlagFinalize | (commit ? kFlagCommit : 0) | pdl_flags(ctx, true, user_flags, s, mine, n_mine, 0);
+    const int rpt = ((user_flags & EGPU_F_INPUTS_READY) && ctx->D <= 16) ? kRowsPerThreadPipelined : kRowsPerThread;
+    const int64_t want = single_ctas(ctx, kern, R, rpt, true);
+    if (want == 0) return EGPU_ERR_INVALID;
+    rc = launch_pdl(ctx, kern, want, s, ctx->d_state, d_rc, d_rm, static_cast<long long>(R), d_idx, d_cards, d_delta, d_table_out,
+                    flags, static_cast<unsigned long long>(ctx->seq % kEpiSlots));
     if (rc != EGPU_OK) return rc;
     ctx->seq += 1;
     note_scan(ctx, s, mine, n_mine, commit, 0);
@@ -530,6 +568,46 @@ int ensure_staging(egpu_ctx* ctx, int64_t rows) {
     return EGPU_OK;
 }
 
+// host-buffer entry points: the requests into the staging arrays ...
+int stage_requests(egpu_ctx* ctx, const int32_t* req_core, const int32_t* req_mem, int64_t R, cudaStream_t s) {
+    const int rc = ensure_staging(ctx, R > 0 ? R : 1);
+    if (rc != EGPU_OK) return rc;
+    if (R > 0) {
+        EGPU_CUDA(ctx, cudaMemcpyAsync(ctx->d_req_core, req_core, sizeof(int32_t) * R, cudaMemcpyHostToDevice, s));
+        EGPU_CUDA(ctx, cudaMemcpyAsync(ctx->d_req_mem, req_mem, sizeof(int32_t) * R, cudaMemcpyHostToDevice, s));
+    }
+    return EGPU_OK;
+}
+// ... and the indices and demand sums back; waits for the stream
+int unstage_results(egpu_ctx* ctx, int32_t* out_idx, int64_t R, cudaStream_t s) {
+    if (R > 0) EGPU_CUDA(ctx, cudaMemcpyAsync(out_idx, ctx->d_idx, sizeof(int32_t) * R, cudaMemcpyDeviceToHost, s));
+    EGPU_CUDA(ctx, cudaMemcpyAsync(ctx->h_delta, ctx->d_delta, sizeof(long long) * 2 * ctx->D, cudaMemcpyDeviceToHost, s));
+    EGPU_CUDA(ctx, cudaStreamSynchronize(s));
+    return EGPU_OK;
+}
+
+// Grow-only arena of the replays: the events (kind, a, b) copied in, the int32 indices out
+// (ev[0..3]), then `extra` bytes (*extra).  No cudaMalloc/cudaFree on the call path once grown.
+int replay_stage(egpu_ctx* ctx, const int32_t* kind, const int32_t* a, const int32_t* b, int64_t E, size_t extra, cudaStream_t s,
+                 int32_t** ev, char** extra_out) {
+    const size_t ebytes = (sizeof(int32_t) * static_cast<size_t>(E) + 255) & ~static_cast<size_t>(255);
+    const size_t need = 4 * ebytes + extra;
+    if (need > ctx->arena_cap) {
+        if (ctx->arena) cudaFree(ctx->arena);
+        ctx->arena = nullptr;
+        ctx->arena_cap = 0;
+        EGPU_CUDA(ctx, cudaMalloc(&ctx->arena, need + need / 4));
+        ctx->arena_cap = need + need / 4;
+    }
+    char* base = static_cast<char*>(ctx->arena);
+    for (int j = 0; j < 4; ++j) ev[j] = reinterpret_cast<int32_t*>(base + j * ebytes);
+    *extra_out = extra ? base + 4 * ebytes : nullptr;
+    EGPU_CUDA(ctx, cudaMemcpyAsync(ev[0], kind, sizeof(int32_t) * E, cudaMemcpyHostToDevice, s));
+    EGPU_CUDA(ctx, cudaMemcpyAsync(ev[1], a, sizeof(int32_t) * E, cudaMemcpyHostToDevice, s));
+    EGPU_CUDA(ctx, cudaMemcpyAsync(ev[2], b, sizeof(int32_t) * E, cudaMemcpyHostToDevice, s));
+    return EGPU_OK;
+}
+
 bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 
 // device-visible alias of a pinned (mapped) host allocation, nullptr for anything else
@@ -546,7 +624,7 @@ void* mapped_alias(const void* p) {
 
 extern "C" {
 
-int egpu_abi_version(void) { return 1004; }  // 1.4: + multi-batch launches, stateless query, start gate (additive)
+int egpu_abi_version(void) { return 1005; }  // 1.5: + whole-card requests: egpu_bestfit_cards[_dev], egpu_replay_cards (additive)
 
 const char* egpu_strerror(int code) {
     switch (code) {
@@ -630,6 +708,7 @@ void egpu_ctx_destroy(egpu_ctx* ctx) {
     cudaFree(ctx->d_req_core);
     cudaFree(ctx->d_req_mem);
     cudaFree(ctx->d_idx);
+    cudaFree(ctx->d_cards);
     cudaFree(ctx->d_delta);
     cudaFree(ctx->d_table_out);
     if (ctx->h_delta) cudaFreeHost(ctx->h_delta);
@@ -914,20 +993,14 @@ int egpu_bestfit_batch(egpu_ctx* ctx, const int32_t* req_core, const int32_t* re
         if (rc != EGPU_OK) return rc;
         EGPU_CUDA(ctx, cudaStreamSynchronize(s));
     } else {
-        rc = ensure_staging(ctx, R > 0 ? R : 1);
+        rc = stage_requests(ctx, req_core, req_mem, R, s);
         if (rc != EGPU_OK) return rc;
-        if (R > 0) {
-            EGPU_CUDA(ctx, cudaMemcpyAsync(ctx->d_req_core, req_core, sizeof(int32_t) * R, cudaMemcpyHostToDevice, s));
-            EGPU_CUDA(ctx, cudaMemcpyAsync(ctx->d_req_mem, req_mem, sizeof(int32_t) * R, cudaMemcpyHostToDevice, s));
-        }
         rc = prefix ? launch_prefix_commit(ctx, ctx->d_req_core, ctx->d_req_mem, R, ctx->d_idx, ctx->d_delta, nullptr,
                                            (commit & EGPU_F_COMMIT) ? EGPU_F_COMMIT : 0, s)
                     : launch_snapshot(ctx, ctx->d_req_core, ctx->d_req_mem, R, ctx->d_idx, ctx->d_delta, nullptr,
                                       (commit & EGPU_F_COMMIT) ? EGPU_F_COMMIT : 0, s);
+        if (rc == EGPU_OK) rc = unstage_results(ctx, out_idx, R, s);
         if (rc != EGPU_OK) return rc;
-        if (R > 0) EGPU_CUDA(ctx, cudaMemcpyAsync(out_idx, ctx->d_idx, sizeof(int32_t) * R, cudaMemcpyDeviceToHost, s));
-        EGPU_CUDA(ctx, cudaMemcpyAsync(ctx->h_delta, ctx->d_delta, sizeof(long long) * 2 * D, cudaMemcpyDeviceToHost, s));
-        EGPU_CUDA(ctx, cudaStreamSynchronize(s));
     }
     if (out_delta_core) std::memcpy(out_delta_core, ctx->h_delta, sizeof(int64_t) * D);
     if (out_delta_mem) std::memcpy(out_delta_mem, ctx->h_delta + D, sizeof(int64_t) * D);
@@ -1218,22 +1291,13 @@ int egpu_replay(egpu_ctx* ctx, const int32_t* kind, const int32_t* a, const int3
     // staging comes from the context's grow-only arena (three inputs, one output, the `live`
     // map when it does not fit in shared memory): no cudaMalloc/cudaFree on the call path
     cudaStream_t s = ctx->stream;
-    const size_t ebytes = (sizeof(int32_t) * static_cast<size_t>(E) + 255) & ~static_cast<size_t>(255);
     const size_t lbytes = E > kReplaySmemEvents ? ((static_cast<size_t>(E) + 255) & ~static_cast<size_t>(255)) : 0;
-    const size_t need = 4 * ebytes + lbytes;
-    if (need > ctx->arena_cap) {
-        if (ctx->arena) cudaFree(ctx->arena);
-        ctx->arena = nullptr;
-        ctx->arena_cap = 0;
-        EGPU_CUDA(ctx, cudaMalloc(&ctx->arena, need + need / 4));
-        ctx->arena_cap = need + need / 4;
-    }
-    char* base = static_cast<char*>(ctx->arena);
-    int32_t* d_kind = reinterpret_cast<int32_t*>(base);
-    int32_t* d_a = reinterpret_cast<int32_t*>(base + ebytes);
-    int32_t* d_b = reinterpret_cast<int32_t*>(base + 2 * ebytes);
-    int32_t* d_out = reinterpret_cast<int32_t*>(base + 3 * ebytes);
-    signed char* d_live = lbytes ? reinterpret_cast<signed char*>(base + 4 * ebytes) : nullptr;
+    int32_t* ev[4];
+    char* extra = nullptr;
+    const int rc = replay_stage(ctx, kind, a, b, E, lbytes, s, ev, &extra);
+    if (rc != EGPU_OK) return rc;
+    int32_t *d_kind = ev[0], *d_a = ev[1], *d_b = ev[2], *d_out = ev[3];
+    signed char* d_live = reinterpret_cast<signed char*>(extra);
     size_t smem = 0;
     if (E <= kReplaySmemEvents) {
         smem = static_cast<size_t>((E + 15) & ~15ll);
@@ -1242,9 +1306,6 @@ int egpu_replay(egpu_ctx* ctx, const int32_t* kind, const int32_t* a, const int3
             ctx->replay_configured = true;
         }
     }
-    EGPU_CUDA(ctx, cudaMemcpyAsync(d_kind, kind, sizeof(int32_t) * E, cudaMemcpyHostToDevice, s));
-    EGPU_CUDA(ctx, cudaMemcpyAsync(d_a, a, sizeof(int32_t) * E, cudaMemcpyHostToDevice, s));
-    EGPU_CUDA(ctx, cudaMemcpyAsync(d_b, b, sizeof(int32_t) * E, cudaMemcpyHostToDevice, s));
     ctx->prev_is_scan = false;
     ctx->lut_dirty = true;
     if (ctx->D <= 32 && E <= kReplaySmemEvents) {
@@ -1261,6 +1322,80 @@ int egpu_replay(egpu_ctx* ctx, const int32_t* kind, const int32_t* a, const int3
     EGPU_CUDA(ctx, cudaGetLastError());
     ctx->launches += 1;
     EGPU_CUDA(ctx, cudaMemcpyAsync(out_idx, d_out, sizeof(int32_t) * E, cudaMemcpyDeviceToHost, s));
+    EGPU_CUDA(ctx, cudaStreamSynchronize(s));
+    return EGPU_OK;
+}
+
+int egpu_bestfit_cards_dev(egpu_ctx* ctx, const int32_t* d_req_core, const int32_t* d_req_mem, int64_t R, int32_t* d_out_idx,
+                           uint64_t* d_out_cards, int64_t* d_delta, int32_t* d_table_out, int flags, void* stream) {
+    if (!ctx || R < 0 || R > kMaxRows || (flags & ~(EGPU_F_COMMIT | EGPU_F_INPUTS_READY))) return EGPU_ERR_INVALID;
+    if (R > 0 && (!d_req_core || !d_req_mem || !d_out_idx)) return EGPU_ERR_INVALID;
+    if (!aligned16(d_req_core) || !aligned16(d_req_mem) || !aligned16(d_out_idx) || !aligned16(d_out_cards) ||
+        !aligned16(d_delta) || !aligned16(d_table_out))
+        return EGPU_ERR_INVALID;
+    std::lock_guard<std::mutex> g(ctx->mu);
+    if (!ctx->has_table) return EGPU_ERR_NO_TABLE;
+    EGPU_CUDA(ctx, cudaSetDevice(ctx->dev));
+    cudaStream_t s = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
+    return launch_cards(ctx, d_req_core, d_req_mem, R, d_out_idx, reinterpret_cast<unsigned long long*>(d_out_cards),
+                        reinterpret_cast<long long*>(d_delta), d_table_out, flags, s);
+}
+
+int egpu_bestfit_cards(egpu_ctx* ctx, const int32_t* req_core, const int32_t* req_mem, int64_t R, int32_t* out_idx,
+                       uint64_t* out_cards, int64_t* out_delta_core, int64_t* out_delta_mem, int commit) {
+    if (!ctx || R < 0 || R > kMaxRows || (commit & ~EGPU_F_COMMIT)) return EGPU_ERR_INVALID;
+    if (R > 0 && (!req_core || !req_mem || !out_idx)) return EGPU_ERR_INVALID;
+    std::lock_guard<std::mutex> g(ctx->mu);
+    if (!ctx->has_table) return EGPU_ERR_NO_TABLE;
+    EGPU_CUDA(ctx, cudaSetDevice(ctx->dev));
+    cudaStream_t s = ctx->stream;
+    int rc = stage_requests(ctx, req_core, req_mem, R, s);
+    if (rc != EGPU_OK) return rc;
+    if (out_cards && R > ctx->d_cards_cap) {
+        cudaFree(ctx->d_cards);
+        ctx->d_cards = nullptr;
+        ctx->d_cards_cap = 0;
+        EGPU_CUDA(ctx, cudaMalloc(&ctx->d_cards, sizeof(unsigned long long) * ctx->d_cap_rows));
+        ctx->d_cards_cap = ctx->d_cap_rows;
+    }
+    unsigned long long* d_cards = out_cards ? ctx->d_cards : nullptr;
+    rc = launch_cards(ctx, ctx->d_req_core, ctx->d_req_mem, R, ctx->d_idx, d_cards, ctx->d_delta, nullptr, commit, s);
+    if (rc != EGPU_OK) return rc;
+    if (d_cards && R > 0)
+        EGPU_CUDA(ctx, cudaMemcpyAsync(out_cards, d_cards, sizeof(unsigned long long) * R, cudaMemcpyDeviceToHost, s));
+    rc = unstage_results(ctx, out_idx, R, s);
+    if (rc != EGPU_OK) return rc;
+    if (out_delta_core) std::memcpy(out_delta_core, ctx->h_delta, sizeof(int64_t) * ctx->D);
+    if (out_delta_mem) std::memcpy(out_delta_mem, ctx->h_delta + ctx->D, sizeof(int64_t) * ctx->D);
+    return EGPU_OK;
+}
+
+int egpu_replay_cards(egpu_ctx* ctx, const int32_t* kind, const int32_t* a, const int32_t* b, int64_t E, int32_t* out_idx,
+                      uint64_t* out_cards) {
+    if (!ctx || E < 0 || E > 0x7fffffffll) return EGPU_ERR_INVALID;
+    if (E > 0 && (!kind || !a || !b || !out_idx)) return EGPU_ERR_INVALID;
+    std::lock_guard<std::mutex> g(ctx->mu);
+    if (!ctx->has_table) return EGPU_ERR_NO_TABLE;
+    if (E == 0) return EGPU_OK;
+    EGPU_CUDA(ctx, cudaSetDevice(ctx->dev));
+    cudaStream_t s = ctx->stream;
+    // after the four event arrays: the card masks out, then every ALLOC's cards and first card
+    const size_t mbytes = (sizeof(unsigned long long) * static_cast<size_t>(E) + 255) & ~static_cast<size_t>(255);
+    int32_t* ev[4];
+    char* extra = nullptr;
+    const int rc = replay_stage(ctx, kind, a, b, E, 2 * mbytes + static_cast<size_t>(E), s, ev, &extra);
+    if (rc != EGPU_OK) return rc;
+    unsigned long long* d_cards = reinterpret_cast<unsigned long long*>(extra);
+    unsigned long long* d_live = reinterpret_cast<unsigned long long*>(extra + mbytes);
+    signed char* d_live_idx = reinterpret_cast<signed char*>(extra + 2 * mbytes);
+    ctx->prev_is_scan = false;
+    ctx->lut_dirty = true;
+    replay_cards_kernel<<<1, 32, 0, s>>>(ctx->d_state, ev[0], ev[1], ev[2], E, ev[3], out_cards ? d_cards : nullptr, d_live,
+                                         d_live_idx);
+    EGPU_CUDA(ctx, cudaGetLastError());
+    ctx->launches += 1;
+    EGPU_CUDA(ctx, cudaMemcpyAsync(out_idx, ev[3], sizeof(int32_t) * E, cudaMemcpyDeviceToHost, s));
+    if (out_cards) EGPU_CUDA(ctx, cudaMemcpyAsync(out_cards, d_cards, sizeof(unsigned long long) * E, cudaMemcpyDeviceToHost, s));
     EGPU_CUDA(ctx, cudaStreamSynchronize(s));
     return EGPU_OK;
 }

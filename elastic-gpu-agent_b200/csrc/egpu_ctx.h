@@ -19,6 +19,9 @@ using SingleFn = void (*)(DevState*, const int32_t*, const int32_t*, long long, 
                           unsigned long long, const DevLut*, unsigned long long*);
 using MultiFn = void (*)(DevState*, const MultiArgs, int, int, unsigned int, unsigned long long, const DevLut*);
 using PackedFn = void (*)(DevState*, const uint32_t*, long long, signed char*, long long*, int32_t*, int, unsigned long long);
+// whole-card requests (cards_scan_kernel): one batch, indices and optional card masks
+using CardsFn = void (*)(DevState*, const int32_t*, const int32_t*, long long, int32_t*, unsigned long long*, long long*,
+                         int32_t*, int, unsigned long long);
 
 template <class Fn>
 struct ScanKernel {
@@ -37,6 +40,7 @@ struct egpu_ctx {
     ScanKernel<SingleFn> single[kSingleForms][kDBuckets];
     ScanKernel<MultiFn> multi[2][kDBuckets];  // [0 = register scan, 1 = lookup scan]
     ScanKernel<PackedFn> packed[kDBuckets];
+    ScanKernel<CardsFn> cards[kDBuckets];
     void* h_qtable = nullptr;         // pinned host image of that table (the part of DevState before `peer`)
     DevState* d_qstate = nullptr;     // scratch table of egpu_bestfit_query (the context's own table is not touched)
     unsigned long long* h_gate = nullptr;      // pinned: start gates the host has opened (egpu_peer_gate_open)
@@ -70,6 +74,8 @@ struct egpu_ctx {
     long long* h_delta = nullptr;     // pinned
     long long* h_delta_dev = nullptr; // its device-visible alias
     int32_t* h_table = nullptr;       // pinned int32[3*64]
+    unsigned long long* d_cards = nullptr;  // card masks of egpu_bestfit_cards (grow-only)
+    int64_t d_cards_cap = 0;
     bool replay_configured = false;   // shared-memory opt-in of the replay kernels done
     // bookkeeping for programmatic dependent launch (see pdl_flags)
     bool prev_is_scan = false;        // the last kernel this context launched was a snapshot scan ...

@@ -227,7 +227,7 @@ __device__ __forceinline__ void epilogue_publish(const unsigned long long* wacc,
         // rank.  Only the oversubscription flag needs both sums of a device: the two finishers swap
         // their sign bits through ep.pair[d] (the second one to come writes the flag).  Critical
         // path of a launch's last CTA: one L2 round trip (two with table'), against red + fence +
-        // ticket + re-load in the general path below.  Sums < 2^49 (EGPU_MAX_ROWS rows of < 2^18).
+        // ticket + re-load in the general path below.  Sums < 2^49 (EGPU_MAX_ROWS rows of < 2^18; a whole-card row of spec 2.8 adds < 2^18 to each of its cards, so that holds).
         if (tid >= 2 * D) return;
         const int d = tid < D ? tid : tid - D;
         const int j = tid < D ? core_off + tid : mem_off + (tid - D);

@@ -367,6 +367,46 @@ int egpu_synth_requests_dev(egpu_ctx* ctx, int dist, uint64_t seed,
 int egpu_replay(egpu_ctx* ctx, const int32_t* kind, const int32_t* a,
                 const int32_t* b, int64_t E, int32_t* out_idx);
 
+/* ---- whole-card requests (DESIGN.md §2.8) ------------------------------- */
+
+/* A container asking for more than 100 gpu-core units gets whole GPUs:
+ * core = 100*k with 2 <= k <= 64 asks for k cards with free_core = 100 and
+ * free_mem >= mem each, and every card gives (100, mem) - memory is per card.
+ * The k cards are the k best fits of (100, mem), i.e. what k sequential best-fit
+ * picks give.  Any other core > 100 (not a multiple of 100, k > 64, or k > D)
+ * is infeasible.  core <= 100 is the single-card rule of egpu_bestfit_batch /
+ * egpu_replay, unchanged: on batches without whole-card rows these entry points
+ * compute exactly what those do.
+ *   out_idx[r]    the first card, the tightest one (not necessarily the lowest
+ *                 index), or -1
+ *   out_cards[r]  mask of every card the row holds (1 << idx for a single-card
+ *                 row, 0 when infeasible); may be NULL, then no mask is stored
+ *                 (12 bytes of traffic per request instead of 20)
+ * Demand sums, table', commit and the sticky oversubscription flag are those of
+ * egpu_bestfit_batch[_dev] with every card of a row adding (100, mem) to its own
+ * device.  These entry points always run the register scan: egpu_set_variant
+ * does not apply to them.
+ * egpu_bestfit_cards: host buffers, commit = 0 or EGPU_F_COMMIT.
+ * egpu_bestfit_cards_dev: as egpu_bestfit_batch_dev; flags = EGPU_F_COMMIT |
+ * EGPU_F_INPUTS_READY (EGPU_F_PREFIX_COMMIT and any other flag are
+ * EGPU_ERR_INVALID); every device array, d_out_cards, d_delta and d_table_out
+ * included, must be 16-byte aligned; pipelines with the other scans of the
+ * context under the same rules. */
+int egpu_bestfit_cards(egpu_ctx* ctx, const int32_t* req_core, const int32_t* req_mem, int64_t R,
+                       int32_t* out_idx, uint64_t* out_cards, int64_t* out_delta_core,
+                       int64_t* out_delta_mem, int commit);
+int egpu_bestfit_cards_dev(egpu_ctx* ctx, const int32_t* d_req_core, const int32_t* d_req_mem,
+                           int64_t R, int32_t* d_out_idx, uint64_t* d_out_cards, int64_t* d_delta,
+                           int32_t* d_table_out, int flags, void* stream);
+
+/* egpu_replay with whole-card ALLOCs: ALLOC(100*k, mem) takes its k cards on
+ * the current table and subtracts (100, mem) from each; a FREE of a live
+ * whole-card ALLOC gives (100, mem) back to every card it holds and reports that
+ * ALLOC's idx and card mask.  Every other rule is egpu_replay's.  out_cards
+ * (may be NULL) = the cards of each event, 0 for -1. */
+int egpu_replay_cards(egpu_ctx* ctx, const int32_t* kind, const int32_t* a, const int32_t* b,
+                      int64_t E, int32_t* out_idx, uint64_t* out_cards);
+
 #ifdef __cplusplus
 }
 #endif
